@@ -332,6 +332,14 @@ def shim_rate(pt, geoms, mats, cam, calls=1000, warm=32):
         compat.reset()
 
 
+def dump_outputs(out_dir, ctx, live):
+    """What a caller of the timed path receives after its last step (rank 0; with N ranks the image is the reduced one):
+    the summed radiance image (download_sum, 800*800 x 3 float32, 7.7 MB) and the live paths per depth (counters)."""
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "image_sum.npy"), ctx.download_sum())
+    np.save(os.path.join(out_dir, "live_per_depth.npy"), live[:DEPTH].astype(np.float64))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -343,7 +351,14 @@ def main():
     ap.add_argument("--strong-spp", type=int, default=STRONG_SPP, help="total samples of the 4K strong-scaling leg (0 = skip)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the strong leg, the other configs and the shim rate")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed to DIR/<name>.npy (the inputs are fixed and seeded, so "
+                         "two builds can be compared output for output)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -418,6 +433,8 @@ def main():
     segs_all, paths_all, launches_all = (float(x) for x in tot.tolist())
     ms_per_step = ms / args.steps
     value = segs_all / (ms_per_step * 1e-3) / 1e6
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, ctx, live)
 
     # ---- end to end through the host API: H2D scene + render + D2H image, every step ----
     host_img = torch.empty((npix, 3), dtype=torch.float32).pin_memory()

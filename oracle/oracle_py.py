@@ -103,21 +103,25 @@ class OrScene(C.Structure):
     ]
 
 
+# a checkout of CIS565-Fall-2014/Project3-Pathtracer; oracle/_ref is built from it wherever it is present
+REF_DIR = os.environ.get("PT_REFERENCE_DIR") or "/root/reference"
+
+
 def build_oracle(force=False):
-    """Compile the C restatement (and oracle/_ref when /root/reference is present)."""
+    """Compile the C restatement (and oracle/_ref when the reference checkout REF_DIR is present)."""
     if force or not os.path.exists(ORACLE_SO) or os.path.getmtime(ORACLE_SO) < os.path.getmtime(
         os.path.join(HERE, "pt_oracle.c")
     ):
         subprocess.check_call(["make", "-s", "-C", HERE, "oracle"])
-    if os.path.isdir("/root/reference/src"):
+    if os.path.isdir(os.path.join(REF_DIR, "src")):
         srcs = [os.path.join(HERE, "ref_shim.cu"), os.path.join(HERE, "ref_scene_shim.cpp"), os.path.join(HERE, "ref_kernel_shim.cu")]
         if force or not os.path.exists(REF_SO) or os.path.getmtime(REF_SO) < max(os.path.getmtime(s) for s in srcs):
-            subprocess.check_call(["make", "-s", "-C", HERE, "ref"])
+            subprocess.check_call(["make", "-s", "-C", HERE, "ref", "REF=" + REF_DIR])
         # the drop-in build test: a host compiled against the reference's own headers, linked with libpt_b200.so
         dropin, main = os.path.join(HERE, "_ref", "ref_dropin"), os.path.join(HERE, "ref_dropin_main.cpp")
         lib = os.path.join(os.path.dirname(HERE), "project3-pathtracer_b200", "libpt_b200.so")
         if os.path.exists(lib) and (force or not os.path.exists(dropin) or os.path.getmtime(dropin) < os.path.getmtime(main)):
-            subprocess.check_call(["make", "-s", "-C", HERE, "dropin"])
+            subprocess.check_call(["make", "-s", "-C", HERE, "dropin", "REF=" + REF_DIR])
 
 
 def _f32(a):

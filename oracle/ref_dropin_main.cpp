@@ -1,7 +1,7 @@
 // TEST INFRASTRUCTURE ONLY -- proves the drop-in claim of INTEGRATION.md section 1 by building it.
 //
 // A headless host program compiled against the REFERENCE'S OWN headers (src/scene.h, src/sceneStructs.h,
-// src/raytraceKernel.h, src/image.h, src/utilities.h, included from where they lie under /root/reference) and linked
+// src/raytraceKernel.h, src/image.h, src/utilities.h, included from where they lie under the reference checkout) and linked
 // with the reference's own scene.cpp / utilities.cpp / image.cpp / stb_image_write.c -- but NOT with its
 // raytraceKernel.cu: the symbol cudaRaytraceCore(uchar4*, camera*, int, int, material*, int, geom*, int) declared at
 // src/raytraceKernel.h:17 is resolved by libpt_b200.so.  What the program does is what the reference's application does

@@ -1,7 +1,7 @@
 // TEST INFRASTRUCTURE ONLY -- never linked into, loaded by, or shipped with the product.
 //
 // oracle/_ref/libptref_gpu.so: the reference's OWN render entry and kernels -- src/raytraceKernel.cu, included from
-// where it lies under /root/reference (nothing is copied) -- compiled for sm_100a.  Its kernels are the TODO stubs the
+// where it lies under the reference checkout (nothing is copied) -- compiled for sm_100a.  Its kernels are the TODO stubs the
 // reference ships: raytraceRay writes per-pixel noise (src/raytraceKernel.cu:93-104, generateRandomNumberFromThread
 // :29-36), sendImageToPBO converts the image to 8 bits (:58-89).  Running it on the GPU box gives the outputs of the
 // reference ITSELF for the pieces it does implement:

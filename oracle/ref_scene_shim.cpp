@@ -1,7 +1,7 @@
 // TEST INFRASTRUCTURE ONLY -- never linked into, loaded by, or shipped with the product.
 //
 // extern "C" wrappers around the reference's own scene loader and image writer, compiled
-// from /root/reference/src/{scene,utilities,image}.cpp and external stb_image_write.c where
+// from the reference checkout's src/{scene,utilities,image}.cpp and external stb_image_write.c where
 // they lie (see oracle/Makefile).  Used by oracle/gen_golden.py and by the in-container
 // pinning tests.  Reference entry points wrapped:
 //   scene::scene(string)            src/scene.cpp:11-35

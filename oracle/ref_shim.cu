@@ -1,7 +1,7 @@
 // TEST INFRASTRUCTURE ONLY -- never linked into, loaded by, or shipped with the product.
 //
 // oracle/_ref/libptref.so: the reference's OWN __host__ __device__ functions, compiled
-// for the host by nvcc from the sources where they lie under /root/reference (nothing is
+// for the host by nvcc from the sources where they lie under the reference checkout (nothing is
 // copied into this repo).  This file only adds extern "C" batch wrappers so that Python
 // (ctypes) can call them.  It is used for exactly two things:
 //   1. oracle/gen_golden.py  -> writes tests/golden/*.json (the committed golden vectors)

@@ -50,19 +50,30 @@ def _locked():
         os.close(fd)
 
 
+def _stale_outputs(force=False):
+    """(cu sources, cpp sources, library stale, driver stale): the one rule for what a build has to redo"""
+    cu, cpp = _sources()
+    hdr = glob.glob(os.path.join(CSRC, "*.h")) + glob.glob(os.path.join(CSRC, "*.cuh")) + glob.glob(
+        os.path.join(ROOT, "include", "*.h"))
+    lib = force or _stale(LIB, cu + cpp + hdr + [os.path.abspath(__file__)])
+    main = os.path.join(CSRC, "pt_main.cpp")
+    driver = os.path.exists(main) and (lib or _stale(DRIVER, [main, LIB]))
+    return cu, cpp, lib, driver
+
+
 def build(force=False, verbose=False):
     """Build what is stale.  Serialised by a file lock; outputs are written to a temporary name and renamed, so a
-    concurrent dlopen never sees a half-written file."""
+    concurrent dlopen never sees a half-written file.  An up-to-date build takes no lock and writes nothing, so a
+    built tree can be used read-only."""
+    if not any(_stale_outputs(force)[2:]):
+        return LIB
     with _locked():
         return _build(force, verbose)
 
 
 def _build(force, verbose):
-    cu, cpp = _sources()
-    hdr = glob.glob(os.path.join(CSRC, "*.h")) + glob.glob(os.path.join(CSRC, "*.cuh")) + glob.glob(
-        os.path.join(ROOT, "include", "*.h"))
-    built = False
-    if force or _stale(LIB, cu + cpp + hdr + [os.path.abspath(__file__)]):
+    cu, cpp, lib, driver = _stale_outputs(force)  # again under the lock: another process may have built meanwhile
+    if lib:
         tmp = LIB + ".tmp.%d" % os.getpid()
         cmd = [nvcc()] + NVCC_FLAGS + (["-Xptxas", "-v"] if verbose else []) + [
             "-I", os.path.join(ROOT, "include"), "-shared", "-o", tmp] + cu + cpp + ["-lz"]
@@ -72,9 +83,8 @@ def _build(force, verbose):
         finally:
             if os.path.exists(tmp):
                 os.remove(tmp)
-        built = True
-    main = os.path.join(CSRC, "pt_main.cpp")
-    if os.path.exists(main) and (force or built or _stale(DRIVER, [main, LIB])):
+    if driver:
+        main = os.path.join(CSRC, "pt_main.cpp")
         tmp = DRIVER + ".tmp.%d" % os.getpid()
         try:
             subprocess.check_call(["g++", "-std=c++17", "-O2", "-pthread", "-I", os.path.join(ROOT, "include"), main, "-o", tmp,

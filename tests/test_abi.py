@@ -30,6 +30,16 @@ def test_library_exports_every_declared_symbol(pt):
     assert lib.pt_abi_version() == 1
 
 
+def test_up_to_date_build_writes_nothing(pt, monkeypatch):
+    """a built tree may be read-only: loading it must not take the build lock (which creates a file in the package)"""
+    pt.lib()
+
+    def no_lock():
+        raise AssertionError("build() took the lock although nothing was stale")
+    monkeypatch.setattr(pt.build, "_locked", no_lock)
+    assert pt.build.build() == pt.LIB_PATH
+
+
 def test_cudaRaytraceCore_symbol_has_the_reference_mangling(pt):
     """same C++ symbol as the reference's src/raytraceKernel.h:17 declaration produces"""
     out = subprocess.check_output(["nm", "-D", "--defined-only", pt.LIB_PATH], text=True)

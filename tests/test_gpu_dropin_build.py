@@ -17,7 +17,7 @@ EXE = os.path.join(ROOT, "oracle", "_ref", "ref_dropin")
 
 def test_reference_host_linked_against_libpt_b200(pt, sample_scene, tmp_path):
     if not os.path.exists(EXE):
-        pytest.skip("oracle/_ref/ref_dropin not built (needs /root/reference at build time: make -C oracle dropin)")
+        pytest.skip("oracle/_ref/ref_dropin not built (needs the reference checkout at build time: PT_REFERENCE_DIR, default /root/reference)")
     depth, seed, iters = 8, 565, 4
     out = tmp_path / "dropin.png"
     pbo = tmp_path / "pbo.raw"

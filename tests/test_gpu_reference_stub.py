@@ -2,10 +2,13 @@
 compiled for sm_100a (oracle/ref_kernel_shim.cu includes it from where it lies).  Its renderer is the stub the
 reference ships, so what can be compared is what it does implement: the per-pixel noise of raytraceRay /
 generateRandomNumberFromThread (:29-36, 93-104) and the 8-bit conversion of sendImageToPBO (:58-89).  Bit-exact."""
+import json
+import os
+
 import numpy as np
 import pytest
 
-from conftest import same_bits, with_resolution
+from conftest import GOLD, f32, same_bits, with_resolution
 
 pytestmark = pytest.mark.gpu
 
@@ -14,7 +17,7 @@ pytestmark = pytest.mark.gpu
 def refgpu():
     from oracle_py import RefGpu
     if not RefGpu.available():
-        pytest.skip("oracle/_ref/libptref_gpu.so not built (needs /root/reference at build time)")
+        pytest.skip("oracle/_ref/libptref_gpu.so not built (needs the reference checkout at build time: PT_REFERENCE_DIR, default /root/reference)")
     return RefGpu()
 
 
@@ -30,6 +33,19 @@ def test_stub_image_equals_the_reference_kernel(pt, oracle, refgpu, W, H, k):
     # the host build of the same function draws in the opposite order; oracle and CUDA agree on both
     assert same_bits(pt.reference_stub_image(W, H, k, pt.STUB_ORDER_HOST), oracle.noise_image(W, H, float(k), True))
     assert same_bits(ours, oracle.noise_image(W, H, float(k), False))
+
+
+def test_stub_image_equals_the_stored_reference_output(pt):
+    """the same comparison against the reference's own output stored in tests/golden/sampling_vectors.json (its host
+    build of generateRandomNumberFromThread), so it runs without a build of the reference"""
+    with open(os.path.join(GOLD, "sampling_vectors.json")) as f:
+        cases = json.load(f)["ref_noise_host"]
+    for k in cases:
+        want = f32(k["rgb"]).reshape(-1, 3)
+        assert same_bits(pt.reference_stub_image(k["W"], k["H"], int(k["time"]), pt.STUB_ORDER_HOST), want)
+        # the device build draws the same three numbers in the opposite order (stored host output only; the device
+        # order itself is compared with the reference's kernel by test_stub_image_equals_the_reference_kernel)
+        assert same_bits(pt.reference_stub_image(k["W"], k["H"], int(k["time"]), pt.STUB_ORDER_DEVICE), want[:, ::-1])
 
 
 def test_resolve_rgba8_equals_sendImageToPBO(pt, refgpu, sample_scene):

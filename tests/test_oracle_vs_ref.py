@@ -6,7 +6,7 @@ import pytest
 from conftest import same_bits
 from oracle_py import Ref
 
-pytestmark = pytest.mark.skipif(not Ref.available(), reason="oracle/_ref not built (needs /root/reference)")
+pytestmark = pytest.mark.skipif(not Ref.available(), reason="oracle/_ref not built (needs the reference checkout at build time: PT_REFERENCE_DIR, default /root/reference)")
 
 
 @pytest.fixture(scope="module")
