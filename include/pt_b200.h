@@ -213,6 +213,16 @@ int pt_selftest_math(int device, uint64_t bad[3]);
  * apart from the path segments.  The shadow rays of a depth are queued (64 bytes each, one queue entry per path of
  * wavefront capacity, allocated by the first render that needs them) and traced by a launch of their own. */
 int pt_set_direct_lighting(pt_context* ctx, int on);
+/* ---- subsurface scattering (calculateScatterAndAbsorption, stub at src/interactions.h:36-39; README.md "subsurface
+ * scattering") ----
+ * Off by default: SCATTER and RSCTCOEFF are then carried but ignored, and every result is unchanged.  On: a sphere / cube
+ * whose material has REFR > 0, SCATTER > 0 and RSCTCOEFF > 0 holds a homogeneous medium -- scattering coefficient
+ * RSCTCOEFF (isotropic phase function), absorption ABSCOEFF per channel, the refractive surface as its boundary.  A
+ * segment that ran inside it ends at a free-flight distance s = -log(1 - u) / RSCTCOEFF if that comes first: the path
+ * goes on from there in a uniform direction, weighted by calculateTransmission over s, and the next emission it meets
+ * counts in full (no light sample at such an event).  Each scattering event is one segment of max_depth.  Media block
+ * shadow rays like any refractive geom; nested or overlapping media are not modelled.  Drops an open sample stream. */
+int pt_set_subsurface(pt_context* ctx, int on);
 /* shadow rays traced by pt_render calls since the last pt_clear; n_lights (may be NULL) = emissive geoms of the scene */
 int pt_shadow_rays(pt_context* ctx, uint64_t* shadow_rays, int* n_lights);
 
@@ -231,6 +241,13 @@ int pt_random_directions_in_sphere(int device, int n, const float* xi1, const fl
  * absorption = n x 3, distance = n.  pt_render applies it to every segment that runs inside a refractive geom whose
  * material has ABSCOEFF > 0. */
 int pt_calculate_transmission(int device, int n, const float* absorption, const float* distance, float* out);
+/* calculateScatterAndAbsorption (stub at src/interactions.h:36-39): the free flight pt_set_subsurface traces, for n
+ * segments of length distance[i] inside a medium with absorption[i] (x3) and scattering coefficient scatter[i] > 0,
+ * driven by u[i] = (xi1, xi2, xf) in [0,1): s[i] = -log(1 - xf) / scatter[i]; if s[i] < distance[i] then scattered[i] = 1,
+ * direction[i] = getRandomDirectionInSphere(xi1, xi2), weight[i] = calculateTransmission over s[i]; otherwise
+ * scattered[i] = 0, direction[i] = 0 and weight[i] = calculateTransmission over distance[i]. */
+int pt_sample_medium(int device, int n, const float* absorption, const float* scatter, const float* distance, const float* u,
+                     int32_t* scattered, float* s, float* direction, float* weight);
 
 /* What the reference's own cudaRaytraceCore leaves in renderCam->image TODAY: its raytraceRay is a stub that overwrites
  * every pixel with generateRandomNumberFromThread(resolution, (float)iterations, x, y) (src/raytraceKernel.cu:29-36,

@@ -193,6 +193,11 @@ class Context:
         """direct light sampling at diffuse bounces (pt_set_direct_lighting); off by default"""
         _check(lib().pt_set_direct_lighting(self._h, C.c_int(1 if on else 0)))
 
+    def set_subsurface(self, on=True):
+        """subsurface scattering inside refractive geoms whose material has SCATTER > 0 and RSCTCOEFF > 0
+        (pt_set_subsurface); off by default"""
+        _check(lib().pt_set_subsurface(self._h, C.c_int(1 if on else 0)))
+
     def shadow_rays(self):
         """(shadow rays traced since the last clear, emissive geoms in the scene)"""
         n, nl = C.c_uint64(), C.c_int()
@@ -285,6 +290,21 @@ def calculate_transmission(absorption, distance, device=0):
     out = np.zeros_like(a)
     _check(lib().pt_calculate_transmission(C.c_int(device), C.c_int(d.size), _p(a), _p(d), _p(out)))
     return out
+
+
+def sample_medium(absorption, scatter, distance, u, device=0):
+    """calculateScatterAndAbsorption (src/interactions.h:36-39), the free flight of subsurface scattering:
+    u = (n, 3) uniforms (xi1, xi2, xf) -> (scattered bool (n,), s (n,), direction (n, 3), weight (n, 3)).
+    s = -log(1 - xf) / scatter; where s < distance the segment scatters there into a uniform direction with weight
+    exp(-absorption * s), elsewhere it passes with direction 0 and weight exp(-absorption * distance)."""
+    a, sc = _arr(absorption, np.float32).reshape(-1, 3), _arr(scatter, np.float32).ravel()
+    d, uu = _arr(distance, np.float32).ravel(), _arr(u, np.float32).reshape(-1, 3)
+    n = d.size
+    assert a.shape[0] == n and sc.size == n and uu.shape[0] == n
+    flag, s = np.zeros(n, np.int32), np.zeros(n, np.float32)
+    dirs, w = np.zeros((n, 3), np.float32), np.zeros((n, 3), np.float32)
+    _check(lib().pt_sample_medium(C.c_int(device), C.c_int(n), _p(a), _p(sc), _p(d), _p(uu), _p(flag), _p(s), _p(dirs), _p(w)))
+    return flag.astype(bool), s, dirs, w
 
 
 STUB_ORDER_DEVICE, STUB_ORDER_HOST = 0, 1

@@ -105,6 +105,10 @@ def set_direct_lighting(on):
     lib().pt_compat_set_direct_lighting(C.c_int(1 if on else 0))
 
 
+def set_subsurface(on):
+    lib().pt_compat_set_subsurface(C.c_int(1 if on else 0))
+
+
 def set_reference_stub(on):
     lib().pt_compat_set_reference_stub(C.c_int(1 if on else 0))
 

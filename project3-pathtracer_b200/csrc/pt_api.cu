@@ -75,6 +75,8 @@ struct pt_context {
   float* d_light_k = nullptr;  // per geom: K = area * n_lights / pi of a light, 0 otherwise
   int n_lights = 0;
   bool nee = false;            // pt_set_direct_lighting
+  bool sss = false;            // pt_set_subsurface
+  int n_media = 0;             // spheres / cubes whose material makes them a scattering medium (DESIGN.md 4)
   float4* d_filt = nullptr;   // kFiltRows arrays of n_pairs float4: filter geometry (pt_filter.cuh)
   int2* d_filt_ids = nullptr;
   FiltSoA filt{};
@@ -118,6 +120,8 @@ struct pt_context {
   int grid_blocks[4] = {0, 0, 0, 0};  // persistent grid per (FIRST,LAST) variant
   int grid_blocks_nee[4] = {0, 0, 0, 0};  // ... of the direct-light-sampling variants
   int grid_blocks_q[2] = {0, 0}, grid_blocks_q_nee[2] = {0, 0};  // k_bounce_q<LAST> (depths >= 1 of the linear mode)
+  int grid_blocks_med[4] = {0, 0, 0, 0}, grid_blocks_med_nee[4] = {0, 0, 0, 0};  // subsurface variants (not LAST: MediumOf)
+  int grid_blocks_q_med = 0, grid_blocks_q_med_nee = 0;                          // ... of k_bounce_q<false>
   size_t q_smem_total = 0;            // k_bounce_q: filter geometry + the warps' candidate queues
   int q_mode = 0;                     // depths >= 1, few geoms: 0 = per depth by the scene's measured survival (h_policy),
                                       // 1 = always k_bounce_q, 2 = always the fused k_bounce (PT_B200_FUSED=1 / =0 force 2 / 1)
@@ -671,41 +675,76 @@ static RaygenConsts make_raygen(const pt_camera_data& c, const pt_lens* lens) {
 // segment cannot carry the no-emission flag either, so <true, true> needs no variant of its own
 template <bool F, bool L>
 struct NeeOf { static constexpr bool value = !(F && L); };
+// the subsurface-scattering variant of LAST: none for the last segment -- a scattering event there ends the path exactly as
+// the refraction it replaces does (neither adds radiance, and no later depth counts the path), so image and live counts
+// are those of the plain kernel
+template <bool L>
+struct MediumOf { static constexpr bool value = !L; };
+
+// resident CTAs per SM of one bounce kernel with `smem` bytes of dynamic shared memory
+template <typename K>
+static int fit_kernel(K kernel, int threads, size_t smem, bool carveout, int* per_sm) {
+  CU(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  if (carveout) CU(cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+  CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(per_sm, kernel, threads, smem));
+  return PT_OK;
+}
 
 template <bool F, bool L>
 static int setup_variant(pt_context* c, int slot) {
-  int per_sm = 0, per_sm_nee = 0;
-  constexpr bool N = NeeOf<F, L>::value;
+  int per_sm = 0, per_sm_nee = 0, per_sm_med = 1, per_sm_med_nee = 1;
+  constexpr bool N = NeeOf<F, L>::value, M = MediumOf<L>::value;
+  int rc;
   if (c->mode) {  // (many geoms: one kernel for every depth, primary rays come from k_raygen_wf)
     CU(cudaFuncSetAttribute(k_bounce_bvh<L>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kBvhSmemBytes));
     CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_bounce_bvh<L>, kBvhThreads, kBvhSmemBytes));
     CU(cudaFuncSetAttribute(k_bounce_bvh<L, N>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kBvhSmemBytes));
     CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm_nee, k_bounce_bvh<L, N>, kBvhThreads, kBvhSmemBytes));
+    if constexpr (M) {
+      if ((rc = fit_kernel(k_bounce_bvh<L, false, true>, kBvhThreads, kBvhSmemBytes, false, &per_sm_med))) return rc;
+      if ((rc = fit_kernel(k_bounce_bvh<L, N, true>, kBvhThreads, kBvhSmemBytes, false, &per_sm_med_nee))) return rc;
+    }
   } else {
     CU(cudaFuncSetAttribute(k_bounce<F, L>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c->smem_bytes));
     CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_bounce<F, L>, kBounceThreads, c->smem_bytes));
     CU(cudaFuncSetAttribute(k_bounce<F, L, N>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c->smem_bytes));
     CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm_nee, k_bounce<F, L, N>, kBounceThreads, c->smem_bytes));
+    if constexpr (M) {
+      if ((rc = fit_kernel(k_bounce<F, L, false, true>, kBounceThreads, c->smem_bytes, false, &per_sm_med))) return rc;
+      if ((rc = fit_kernel(k_bounce<F, L, N, true>, kBounceThreads, c->smem_bytes, false, &per_sm_med_nee))) return rc;
+    }
   }
-  if (per_sm < 1 || per_sm_nee < 1) { pt_set_error_("k_bounce does not fit on an SM"); return PT_ERR_CUDA; }
+  if (per_sm < 1 || per_sm_nee < 1 || per_sm_med < 1 || per_sm_med_nee < 1) { pt_set_error_("k_bounce does not fit on an SM"); return PT_ERR_CUDA; }
   c->grid_blocks[slot] = per_sm * c->sm_count;
   c->grid_blocks_nee[slot] = per_sm_nee * c->sm_count;
+  c->grid_blocks_med[slot] = M ? per_sm_med * c->sm_count : 0;
+  c->grid_blocks_med_nee[slot] = M ? per_sm_med_nee * c->sm_count : 0;
   return PT_OK;
 }
 
 template <bool L>
 static int setup_variant_q(pt_context* c, int slot) {
-  int per_sm = 0, per_sm_nee = 0;
+  int per_sm = 0, per_sm_nee = 0, per_sm_med = 1, per_sm_med_nee = 1;
   constexpr bool N = true;  // (the last segment never samples a light, but it honours the no-emission flag)
+  constexpr bool M = MediumOf<L>::value;
+  int rc;
   CU(cudaFuncSetAttribute(k_bounce_q<L>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c->q_smem_total));
   CU(cudaFuncSetAttribute(k_bounce_q<L>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
   CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_bounce_q<L>, kQThreads, c->q_smem_total));
   CU(cudaFuncSetAttribute(k_bounce_q<L, N>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c->q_smem_total));
   CU(cudaFuncSetAttribute(k_bounce_q<L, N>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
   CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm_nee, k_bounce_q<L, N>, kQThreads, c->q_smem_total));
-  if (per_sm < 1 || per_sm_nee < 1) { pt_set_error_("k_bounce_q does not fit on an SM"); return PT_ERR_CUDA; }
+  if constexpr (M) {
+    if ((rc = fit_kernel(k_bounce_q<L, false, true>, kQThreads, c->q_smem_total, true, &per_sm_med))) return rc;
+    if ((rc = fit_kernel(k_bounce_q<L, N, true>, kQThreads, c->q_smem_total, true, &per_sm_med_nee))) return rc;
+  }
+  if (per_sm < 1 || per_sm_nee < 1 || per_sm_med < 1 || per_sm_med_nee < 1) { pt_set_error_("k_bounce_q does not fit on an SM"); return PT_ERR_CUDA; }
   c->grid_blocks_q[slot] = per_sm * c->sm_count;
   c->grid_blocks_q_nee[slot] = per_sm_nee * c->sm_count;
+  if (M) {
+    c->grid_blocks_q_med = per_sm_med * c->sm_count;
+    c->grid_blocks_q_med_nee = per_sm_med_nee * c->sm_count;
+  }
   return PT_OK;
 }
 
@@ -864,6 +903,12 @@ static int upload_scene(pt_context* c, const pt_static_geom* geoms, int n_geoms,
   CU(cudaMemcpyAsync(c->d_rows, rows.data(), rows.size() * sizeof(float4), cudaMemcpyHostToDevice, c->stream));
   CU(cudaMemcpyAsync(c->d_meta, meta.data(), meta.size() * sizeof(int2), cudaMemcpyHostToDevice, c->stream));
   CU(cudaMemcpyAsync(c->d_mats, mats, (size_t)n_mats * sizeof(pt_material), cudaMemcpyHostToDevice, c->stream));
+  c->n_media = 0;
+  for (int i = 0; i < n_geoms; i++) {
+    if (geoms[i].type > 1) continue;
+    const pt_material& mm = mats[geoms[i].materialid];
+    if (mm.hasRefractive > 0 && mm.hasScatter > 0 && mm.reducedScatterCoefficient > 0) c->n_media++;
+  }
   std::vector<float> geom_k;
   const std::vector<float4> lights = build_lights(geoms, n_geoms, mats, &geom_k);
   if (c->d_light_k) CU(cudaFree(c->d_light_k));
@@ -1095,16 +1140,21 @@ extern "C" int pt_clear(pt_context* c) {
 template <bool F, bool L>
 static cudaError_t launch_bounce(pt_context* c, int slot, const BounceParams& P, uint32_t n_upper, cudaStream_t st) {
   const bool nee = c->nee && c->n_lights > 0 && NeeOf<F, L>::value;
-  constexpr bool N = NeeOf<F, L>::value;
-  uint32_t grid = (uint32_t)(nee ? c->grid_blocks_nee[slot] : c->grid_blocks[slot]);
+  constexpr bool N = NeeOf<F, L>::value, M = MediumOf<L>::value;
+  const bool med = M && c->sss && c->n_media > 0;  // (no medium in the scene: the plain kernels, same results)
+  uint32_t grid = (uint32_t)(med ? (nee ? c->grid_blocks_med_nee[slot] : c->grid_blocks_med[slot])
+                                 : (nee ? c->grid_blocks_nee[slot] : c->grid_blocks[slot]));
   // depths >= 1, few geoms: second half re-batched by winner type -- unless the scene keeps nearly all its paths alive
   // at this depth (closed rooms), where the fused kernel is faster; unknown yet (first wavefronts of a scene): re-batched
   const bool use_q = c->q_mode == 1 || (c->q_mode == 0 && ((volatile int*)c->h_policy)[P.depth] != 2);
   if (!F && !c->mode && use_q) {
-    uint32_t gq = (uint32_t)(nee ? c->grid_blocks_q_nee[L ? 1 : 0] : c->grid_blocks_q[L ? 1 : 0]);
+    uint32_t gq = (uint32_t)(med ? (nee ? c->grid_blocks_q_med_nee : c->grid_blocks_q_med)
+                                 : (nee ? c->grid_blocks_q_nee[L ? 1 : 0] : c->grid_blocks_q[L ? 1 : 0]));
     const uint32_t ctas = (n_upper + kQThreads - 1) / kQThreads;  // one unit per warp at least
     if (ctas < gq) gq = ctas ? ctas : 1;
-    if (nee) k_bounce_q<L, N><<<gq, kQThreads, c->q_smem_total, st>>>(P);
+    if (med && nee) k_bounce_q<L, N, M><<<gq, kQThreads, c->q_smem_total, st>>>(P);
+    else if (med) k_bounce_q<L, false, M><<<gq, kQThreads, c->q_smem_total, st>>>(P);
+    else if (nee) k_bounce_q<L, N><<<gq, kQThreads, c->q_smem_total, st>>>(P);
     else k_bounce_q<L><<<gq, kQThreads, c->q_smem_total, st>>>(P);
   } else if (c->mode) {
     if (F) {  // primary rays into the wavefront's input buffers
@@ -1114,12 +1164,16 @@ static cudaError_t launch_bounce(pt_context* c, int slot, const BounceParams& P,
     }
     const uint32_t ctas = (n_upper + kPoolMin * (kBvhThreads / 32) - 1) / (kPoolMin * (kBvhThreads / 32));  // a (smallest) pool per warp at least
     if (ctas < grid) grid = ctas ? ctas : 1;
-    if (nee) k_bounce_bvh<L, N><<<grid, kBvhThreads, kBvhSmemBytes, st>>>(P);
+    if (med && nee) k_bounce_bvh<L, N, M><<<grid, kBvhThreads, kBvhSmemBytes, st>>>(P);
+    else if (med) k_bounce_bvh<L, false, M><<<grid, kBvhThreads, kBvhSmemBytes, st>>>(P);
+    else if (nee) k_bounce_bvh<L, N><<<grid, kBvhThreads, kBvhSmemBytes, st>>>(P);
     else k_bounce_bvh<L><<<grid, kBvhThreads, kBvhSmemBytes, st>>>(P);
   } else {
     const uint32_t ctas = (n_upper + kBounceThreads - 1) / kBounceThreads;  // one unit per warp at least
     if (ctas < grid) grid = ctas ? ctas : 1;
-    if (nee) k_bounce<F, L, N><<<grid, kBounceThreads, c->smem_bytes, st>>>(P);
+    if (med && nee) k_bounce<F, L, N, M><<<grid, kBounceThreads, c->smem_bytes, st>>>(P);
+    else if (med) k_bounce<F, L, false, M><<<grid, kBounceThreads, c->smem_bytes, st>>>(P);
+    else if (nee) k_bounce<F, L, N><<<grid, kBounceThreads, c->smem_bytes, st>>>(P);
     else k_bounce<F, L><<<grid, kBounceThreads, c->smem_bytes, st>>>(P);
   }
   c->launches++;
@@ -1599,6 +1653,13 @@ extern "C" int pt_set_direct_lighting(pt_context* c, int on) {
   c->nee = on != 0;
   return PT_OK;
 }
+extern "C" int pt_set_subsurface(pt_context* c, int on) {
+  CTX(c);
+  if (int rc = stream_discard(c)) return rc;
+  CU(cudaStreamSynchronize(c->stream));
+  c->sss = on != 0;
+  return PT_OK;
+}
 extern "C" int pt_shadow_rays(pt_context* c, uint64_t* shadow_rays, int* n_lights) {
   CTX(c);
   if (!shadow_rays) { pt_set_error_("shadow_rays is NULL"); return PT_ERR_INVALID; }
@@ -1766,6 +1827,33 @@ extern "C" int pt_calculate_transmission(int device, int n, const float* absorpt
   k_transmission<<<(n + 255) / 256, 256>>>(n, da.p, dd.p, dout.p);
   CU(cudaGetLastError());
   CU(cudaMemcpy(out, dout.p, 3 * (size_t)n * sizeof(float), cudaMemcpyDeviceToHost));
+  return PT_OK;
+}
+
+extern "C" int pt_sample_medium(int device, int n, const float* absorption, const float* scatter, const float* distance,
+                                const float* u, int32_t* scattered, float* s, float* direction, float* weight) {
+  if (n < 0 || (n > 0 && (!absorption || !scatter || !distance || !u || !scattered || !s || !direction || !weight))) {
+    pt_set_error_("bad arguments");
+    return PT_ERR_INVALID;
+  }
+  if (n == 0) return PT_OK;
+  if (int rc = select_device_(device)) return rc;
+  const size_t n3 = 3 * (size_t)n;
+  // one arena: absorption, scatter, distance, u in; s, direction, weight out (floats), then the flags
+  DevBuf<float> buf;
+  CU(buf.alloc(n3 + n + n + n3 + n + n3 + n3 + n));
+  float *da = buf.p, *dsc = da + n3, *dd = dsc + n, *du = dd + n, *ds = du + n3, *ddir = ds + n, *dw = ddir + n3;
+  int32_t* dflag = reinterpret_cast<int32_t*>(dw + n3);
+  CU(cudaMemcpy(da, absorption, n3 * sizeof(float), cudaMemcpyHostToDevice));
+  CU(cudaMemcpy(dsc, scatter, n * sizeof(float), cudaMemcpyHostToDevice));
+  CU(cudaMemcpy(dd, distance, n * sizeof(float), cudaMemcpyHostToDevice));
+  CU(cudaMemcpy(du, u, n3 * sizeof(float), cudaMemcpyHostToDevice));
+  k_sample_medium<<<(n + 255) / 256, 256>>>(n, da, dsc, dd, du, dflag, ds, ddir, dw);
+  CU(cudaGetLastError());
+  CU(cudaMemcpy(scattered, dflag, n * sizeof(int32_t), cudaMemcpyDeviceToHost));
+  CU(cudaMemcpy(s, ds, n * sizeof(float), cudaMemcpyDeviceToHost));
+  CU(cudaMemcpy(direction, ddir, n3 * sizeof(float), cudaMemcpyDeviceToHost));
+  CU(cudaMemcpy(weight, dw, n3 * sizeof(float), cudaMemcpyDeviceToHost));
   return PT_OK;
 }
 

@@ -79,14 +79,6 @@ __device__ __forceinline__ f3 cube_point_th(float4 f0, float4 f1, float4 f2, flo
   return mulMV(f0, f1, f2, p.x, p.y, p.z, 1.0f);
 }
 
-// uniform direction on the unit sphere: z = 1 - 2*xi1, azimuth 2*pi*xi2
-__device__ __forceinline__ f3 sphere_dir(float xi1, float xi2) {
-  const float z = 1.0f - 2.0f * xi1;
-  const float r = sqrt_ieee(fmaxf(0.0f, 1.0f - z * z));
-  float sn, cs;
-  sincos_2pi(xi2, sn, cs);
-  return mk(r * cs, r * sn, z);
-}
 __device__ __forceinline__ f3 sphere_point(float4 f0, float4 f1, float4 f2, float u0, float u1) {
   const f3 d = sphere_dir(u0, u1);
   return mulMV(f0, f1, f2, 0.5f * d.x, 0.5f * d.y, 0.5f * d.z, 1.0f);
@@ -148,6 +140,18 @@ __global__ void k_transmission(int n, const float* absorption, const float* dist
   if (i >= n) return;
   const f3 t = transmission(mk(absorption[3 * i], absorption[3 * i + 1], absorption[3 * i + 2]), distance[i]);
   out[3 * i] = t.x; out[3 * i + 1] = t.y; out[3 * i + 2] = t.z;
+}
+// u = (xi1, xi2, xf) per entry: the three uniforms the renderer takes from the segment's Philox block (u[0], u[1], u[3])
+__global__ void k_sample_medium(int n, const float* absorption, const float* scatter, const float* distance, const float* u,
+                                int32_t* scattered, float* s, float* dir, float* weight) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const MediumSample e = sample_medium(mk(absorption[3 * i], absorption[3 * i + 1], absorption[3 * i + 2]), scatter[i], distance[i],
+                                       u[3 * i], u[3 * i + 1], u[3 * i + 2]);
+  scattered[i] = e.scattered ? 1 : 0;
+  s[i] = e.s;
+  dir[3 * i] = e.dir.x; dir[3 * i + 1] = e.dir.y; dir[3 * i + 2] = e.dir.z;
+  weight[3 * i] = e.weight.x; weight[3 * i + 1] = e.weight.y; weight[3 * i + 2] = e.weight.z;
 }
 
 }  // namespace ptd

@@ -10,6 +10,10 @@
                          (axis-aligned slabs are scaled instead), so it means the same under the reference's radian
                          ROTAT quirk (SURVEY.md D1).
   sample_4k.txt          config 4: sample scene at 3840x2160, 16384 iterations
+  cornell_sss.txt        subsurface scattering (pt_set_subsurface / pt_render sss=1): a closed room with a sphere and a
+                         cube of the sample scene's material 5 coefficients (REFRIOR 2.2, ABSCOEFF .02 5.1 5.7,
+                         RSCTCOEFF 13) with SCATTER 1 -- and RGB 1 1 1, since the sample's RGB 0 0 0 would stop every
+                         path that refracts into them
   procedural(n, seed)    config 3: n spheres/cubes, i.i.d. type, centre, scale, rotation (radians) and material from a
                          fixed seed; written on demand (python scenes/gen_scenes.py --procedural 10000 out.txt)
 """
@@ -116,6 +120,31 @@ def cornell_glass_dof():
     return scene_text(mats, cam, objs, lens=(0.12, 13.0))
 
 
+def cornell_sss():
+    mats = [
+        ((.85, .85, .85), 0, (1, 1, 1), 0, 0, 0, 0, (0, 0, 0), 0, 0),        # 0 white
+        ((.63, .06, .04), 0, (1, 1, 1), 0, 0, 0, 0, (0, 0, 0), 0, 0),        # 1 red
+        ((.15, .48, .09), 0, (1, 1, 1), 0, 0, 0, 0, (0, 0, 0), 0, 0),        # 2 green
+        ((1, 1, 1), 0, (0, 0, 0), 0, 0, 0, 0, (0, 0, 0), 0, 15),             # 3 light
+        ((1, 1, 1), 0, (1, 1, 1), 0, 1, 2.2, 1, (.02, 5.1, 5.7), 13, 0),     # 4 scattering medium
+    ]
+    z0 = (0, 0, 0)
+    objs = [
+        ("cube", 0, [((0, 0, 0), z0, (10, .01, 10))]),      # floor
+        ("cube", 0, [((0, 10, 0), z0, (10, .01, 10))]),     # ceiling
+        ("cube", 0, [((0, 5, -5), z0, (10, 10, .01))]),     # back
+        ("cube", 0, [((0, 5, 5), z0, (10, 10, .01))]),      # front (behind the camera): closed room
+        ("cube", 1, [((-5, 5, 0), z0, (.01, 10, 10))]),     # left
+        ("cube", 2, [((5, 5, 0), z0, (.01, 10, 10))]),      # right
+        ("cube", 3, [((0, 9.9, 0), z0, (3, .15, 3))]),      # emissive panel
+        ("sphere", 4, [((-1.8, 1.6, -1), z0, (3.2, 3.2, 3.2))]),
+        ("cube", 4, [((1.9, 1.25, 0.5), (0, .5, 0), (2.5, 2.5, 2.5))]),  # rotated .5 rad about y
+    ]
+    cam = dict(res=(800, 800), fovy=30, iterations=1024, file="cornell_sss.png",
+               frames=[((0, 5, 4.8), (0, -0.25, -1), (0, 1, 0))])
+    return scene_text(mats, cam, objs)
+
+
 def sample_animated(n_frames=3, res=(800, 800), iterations=5000):
     """the sample scene with a bouncing sphere, a sliding camera and one per-frame array for every object
     (the reference's loader reads `frame k` blocks into per-frame arrays, src/scene.cpp:82-128, and its main loop
@@ -155,7 +184,7 @@ def procedural(n, seed=565, res=(1920, 1080), iterations=1024):
 
 def write_all():
     files = {"sample.txt": sample_scene(), "cornell_glass_dof.txt": cornell_glass_dof(),
-             "sample_4k.txt": sample_scene((3840, 2160), 16384)}
+             "sample_4k.txt": sample_scene((3840, 2160), 16384), "cornell_sss.txt": cornell_sss()}
     for name, text in files.items():
         with open(os.path.join(HERE, name), "w") as f:
             f.write(text)
