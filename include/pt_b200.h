@@ -191,6 +191,18 @@ int pt_intersect_ex(pt_context* ctx, int mode, int n, const float* origin, const
 /* multiply every rounding-error term of the filter's bounds by `scale` (1 = shipped).  Test hook: parity must hold
  * at 1 with margin, i.e. also at scales well below 1; 0 disables the margins. */
 int pt_set_filter_scale(pt_context* ctx, float scale);
+/* Primary rays of a pinhole camera (no lens) in a scene of the pair scan first try a per-pixel candidate, worked out
+ * once per pixel for the whole pixel footprint (DESIGN.md 3a "primary rays"); the filter scan runs only for rays that
+ * candidate does not settle.  The table is rebuilt by pt_context_create, pt_update_scene and pt_set_filter_scale (its
+ * margin scales with the filter's).
+ * pt_primary_hit: the primary ray of each (pixel, sample) pair (as pt_raygen makes it with `seed`) through that depth-0
+ * closest hit, with the results of pt_intersect_ex; decided[i] = 1 if the table's candidate settled ray i.  Scenes of the
+ * pair scan only (PT_ERR_STATE otherwise).
+ * pt_primary_table_info: *active = 1 if the current scene and camera have the table; build_ms (may be NULL) = the time
+ * of one rebuild, measured by rebuilding it. */
+int pt_primary_hit(pt_context* ctx, uint64_t seed, int n, const uint32_t* pixel, const uint32_t* sample, int32_t* geom_id,
+                   float* t, float* point, float* normal, uint8_t* decided, uint64_t* fallbacks);
+int pt_primary_table_info(pt_context* ctx, int* active, float* build_ms);
 /* segments of pt_render calls since the last pt_clear whose closest hit took the exact-scan fallback */
 int pt_filter_stats(pt_context* ctx, uint64_t* fallbacks);
 /* scenes with a hierarchy: segments (and shadow rays) since pt_clear whose nearest candidate was not confirmed by its exact

@@ -228,6 +228,26 @@ class Context:
                                      C.byref(fb)))
         return (gid, t, p, nr, fb.value) if with_stats else (gid, t, p, nr)
 
+    def primary_hit(self, seed, pixel, sample, with_stats=False):
+        """primary rays of (pixel, sample) pairs through depth 0's closest hit -- the per-pixel table's candidate first,
+        then the filter -- -> (geom id, t, point, normal, decided) [+ fallbacks]; decided = the table settled the ray"""
+        pixel, sample = _arr(pixel, np.uint32).ravel(), _arr(sample, np.uint32).ravel()
+        n = pixel.shape[0]
+        gid, t = np.zeros(n, np.int32), np.zeros(n, np.float32)
+        p, nr = np.zeros((n, 3), np.float32), np.zeros((n, 3), np.float32)
+        dec = np.zeros(n, np.uint8)
+        fb = C.c_uint64()
+        _check(lib().pt_primary_hit(self._h, C.c_uint64(seed), C.c_int(n), _p(pixel), _p(sample), _p(gid), _p(t), _p(p),
+                                    _p(nr), _p(dec), C.byref(fb)))
+        out = (gid, t, p, nr, dec.astype(bool))
+        return out + (fb.value,) if with_stats else out
+
+    def primary_table_info(self, time_build=False):
+        """(the current scene and camera have the primary-ray table, ms of one rebuild or None)"""
+        on, ms = C.c_int(), C.c_float()
+        _check(lib().pt_primary_table_info(self._h, C.byref(on), C.byref(ms) if time_build else None))
+        return bool(on.value), (ms.value if time_build else None)
+
     def set_filter_scale(self, scale):
         """test hook: multiply the rounding-error terms of the closest-hit filter's bounds (1 = shipped)"""
         _check(lib().pt_set_filter_scale(self._h, C.c_float(scale)))

@@ -17,6 +17,7 @@
 #include <string>
 #include <algorithm>
 #include <atomic>
+#include <chrono>
 #include <thread>
 #include <functional>
 #include <vector>
@@ -59,6 +60,11 @@ extern "C" int pt_device_count(int* count) {
 }
 
 // ---------------------------------------------------------------- context
+// the filter constants build_filter gave one geom of the pair scan (the primary-ray table is built from them)
+struct FiltGeom {
+  int key, cls, geom;  // key = 2 * pair + half, as the scan reports its candidate
+  float c[3], k[6], wk[6], ew_c, ew_w;
+};
 struct pt_context {
   int device = 0;
   int sm_count = 0;
@@ -87,6 +93,10 @@ struct pt_context {
   BvhSoA bvh{};
   float filter_scale = 1.0f;  // multiplies every error-model term of the filter (test hook; 1 = the shipped bounds)
   std::vector<pt_static_geom> h_geoms;  // host copy, to rebuild the filter when the scale changes
+  std::vector<FiltGeom> filt_geoms;  // the filter constants of every geom (build_filter), for the primary-ray table
+  uint32_t* d_ptab = nullptr;  // per pixel: candidate of the primary rays (k_primary_table), npix words
+  PrimRec* d_prim = nullptr;   // the table's per-geom records (kMaxPrimRecs)
+  bool ptab_on = false;        // d_ptab holds the table of the current scene, camera and filter scale
   GeomSoA g{};
   RaygenConsts cam{};
   uint32_t W = 0, H = 0, npix = 0;
@@ -196,6 +206,7 @@ struct HostFilter {
   std::vector<int2> leaf_meta;
   int root = 0;  // reference of the hierarchy's root: node 0, or the only leaf
   float ew_c_max = 0.0f, ew_w_max = 0.0f;
+  std::vector<FiltGeom> geoms;  // every real geom of the pair scan
 };
 static const int kBvhMinGeoms = 33;  // scenes with fewer geoms use the linear pair scan (shared memory, packed)
 static bool inv3(const double a[3][3], double r[3][3]) {
@@ -429,6 +440,14 @@ static HostFilter build_filter(const pt_static_geom* geoms, int n_geoms, double 
         }
       }
       F.rows.insert(F.rows.end(), r, r + kFiltRows);
+      for (int half = 0; half < (dummy ? 1 : 2); half++) {
+        const Per& z = half ? y : x;
+        FiltGeom e;
+        e.key = 2 * (int)F.ids.size() + half; e.cls = cls; e.geom = z.geom;
+        memcpy(e.c, z.c, sizeof(e.c)); memcpy(e.k, z.k, sizeof(e.k)); memcpy(e.wk, z.wk, sizeof(e.wk));
+        e.ew_c = z.ew_c; e.ew_w = z.ew_w;
+        F.geoms.push_back(e);
+      }
       F.ids.push_back(make_int2(x.geom, y.geom));
     }
     F.end[cls] = (int)F.ids.size();
@@ -827,6 +846,7 @@ static int upload_filter(pt_context* c) {
   c->filt.ids = c->d_filt_ids;
   for (int k = 0; k < kFiltClasses; k++) c->filt.end[k] = F.end[k];
   c->filt.r_scene = F.r_scene;
+  c->filt_geoms = F.geoms;
   // hierarchy
   if (c->d_bvh_nodes) CU(cudaFree(c->d_bvh_nodes));
   if (c->d_bvh_leaves) CU(cudaFree(c->d_bvh_leaves));
@@ -844,6 +864,85 @@ static int upload_filter(pt_context* c) {
     c->bvh.n_leaves = (int)F.leaf_meta.size(); c->bvh.ew_c_max = F.ew_c_max; c->bvh.ew_w_max = F.ew_w_max;
     c->bvh.root = F.root;
   }
+  return PT_OK;
+}
+
+// The primary-ray table (pt_kernels.cuh: k_primary_table, DESIGN.md 3a "primary rays"), for pinhole cameras of
+// pair-scan scenes: one record per filter shape at the eye, in binary64, from the binary32 constants the filter itself
+// uses (each term rounded up), then one device thread per pixel.  Anything that cannot be bounded leaves the table off:
+// depth 0 then runs the filter scan for every ray, exactly as without a table.
+static int build_primary_table(pt_context* c) {
+  c->ptab_on = false;
+  if (c->mode != 0 || c->cam.aperture > 0.0f || c->filt_geoms.empty() || c->filt_geoms.size() > (size_t)kMaxPrimRecs) return PT_OK;
+  const double up = 1.0 + 1e-6;
+  const double o[3] = {c->cam.eye.x, c->cam.eye.y, c->cam.eye.z};
+  const double omax = fmax(fmax(fabs(o[0]), fabs(o[1])), fabs(o[2]));
+  const double w = (4.0 * omax + (double)c->filt.r_scene) * up;  // (make_scan_ray's w, rounding included)
+  std::vector<PrimRec> recs;
+  for (const FiltGeom& e : c->filt_geoms) {
+    if (e.key >= (int)kKeyMask) return PT_OK;
+    PrimRec r;
+    memset(&r, 0, sizeof(r));
+    r.ball = e.cls <= 1;
+    r.key = e.key;
+    double ctr[3], half[3];  // world box around the shape: centre, half extents
+    if (e.cls == 0 || e.cls == 2) {  // world space: the frame is the world translated to the centre
+      double oc2 = 0.0;
+      for (int i = 0; i < 3; i++) {
+        r.A[4 * i] = 1.0;
+        ctr[i] = e.c[i];
+        r.ro[i] = o[i] - ctr[i];
+        r.g[i] = 1.0;
+        oc2 += r.ro[i] * r.ro[i];
+      }
+      if (e.cls == 0) {
+        r.h[0] = sqrt(((double)e.wk[0] + (double)e.wk[1] * w + (double)e.wk[2] * oc2) * up);
+        for (int i = 0; i < 3; i++) half[i] = r.h[0];
+      } else {
+        for (int i = 0; i < 3; i++) half[i] = r.h[i] = ((double)e.wk[i] + (double)e.wk[3 + i] * w) * up;
+      }
+    } else {  // object space
+      const float* A = c->h_geoms[e.geom].inverseTransform;
+      double A3[3][3], Ai[3][3], AtA[3][3], ro2 = 0.0;
+      for (int i = 0; i < 3; i++) {
+        for (int j = 0; j < 3; j++) { A3[i][j] = A[4 * i + j]; r.A[3 * i + j] = A3[i][j]; }
+        r.ro[i] = (double)A[4 * i] * o[0] + (double)A[4 * i + 1] * o[1] + (double)A[4 * i + 2] * o[2] + (double)A[4 * i + 3];
+        ro2 += r.ro[i] * r.ro[i];
+      }
+      if (!inv3(A3, Ai)) return PT_OK;
+      for (int i = 0; i < 3; i++) ctr[i] = -(Ai[i][0] * A[3] + Ai[i][1] * A[7] + Ai[i][2] * A[11]);
+      if (e.cls == 1) {
+        for (int a = 0; a < 3; a++)
+          for (int b = 0; b < 3; b++) { AtA[a][b] = 0.0; for (int k = 0; k < 3; k++) AtA[a][b] += A3[k][a] * A3[k][b]; }
+        double lmin, lmax;
+        sym3_eigen_range(AtA, &lmin, &lmax);
+        r.h[0] = sqrt(((double)e.k[0] + (double)e.k[1] * w + (double)e.k[2] * ro2) * up);
+        r.g[0] = sqrt(fmax(lmax, 0.0)) * 1.001;  // sigma_max(A): a world ball of radius rho fits in an object ball of g rho
+        for (int i = 0; i < 3; i++) half[i] = r.h[0] * sqrt(Ai[i][0] * Ai[i][0] + Ai[i][1] * Ai[i][1] + Ai[i][2] * Ai[i][2]) * 1.001;
+      } else {
+        for (int i = 0; i < 3; i++) {
+          r.h[i] = ((double)e.k[i] + (double)e.k[3 + i] * w) * up;
+          r.g[i] = sqrt(A3[i][0] * A3[i][0] + A3[i][1] * A3[i][1] + A3[i][2] * A3[i][2]) * 1.001;  // |row i of A|
+        }
+        for (int i = 0; i < 3; i++) half[i] = (fabs(Ai[i][0]) * r.h[0] + fabs(Ai[i][1]) * r.h[1] + fabs(Ai[i][2]) * r.h[2]) * 1.001;
+      }
+    }
+    double D2 = 0.0;
+    for (int i = 0; i < 3; i++) { const double q = fabs(o[i] - ctr[i]) + half[i]; D2 += q * q; }
+    r.D = sqrt(D2) * 1.001;
+    r.ew = ((double)e.ew_c + (double)e.ew_w * w) * up;
+    bool finite = std::isfinite(r.D) && std::isfinite(r.ew);
+    for (int i = 0; i < 3; i++) finite = finite && std::isfinite(r.ro[i]) && std::isfinite(r.h[i]) && std::isfinite(r.g[i]);
+    if (!finite) return PT_OK;
+    recs.push_back(r);
+  }
+  if (!c->d_ptab) CU(cudaMalloc(&c->d_ptab, (size_t)c->npix * sizeof(uint32_t)));
+  if (!c->d_prim) CU(cudaMalloc(&c->d_prim, (size_t)kMaxPrimRecs * sizeof(PrimRec)));
+  CU(cudaMemcpyAsync(c->d_prim, recs.data(), recs.size() * sizeof(PrimRec), cudaMemcpyHostToDevice, c->stream));
+  k_primary_table<<<(c->npix + 127) / 128, 128, 0, c->stream>>>(c->cam, c->d_prim, (int)recs.size(), (double)c->filter_scale, c->d_ptab);
+  CU(cudaGetLastError());
+  CU(cudaStreamSynchronize(c->stream));  // recs dies at return
+  c->ptab_on = true;
   return PT_OK;
 }
 
@@ -951,8 +1050,9 @@ static int upload_scene(pt_context* c, const pt_static_geom* geoms, int n_geoms,
       if ((rc = setup_variant_q<true>(c, 1))) return rc;
     }
     CU(cudaFuncSetAttribute(k_intersect_list, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c->geom_smem));
+    CU(cudaFuncSetAttribute(k_primary_list, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c->geom_smem));
   }
-  return PT_OK;
+  return build_primary_table(c);
 }
 
 // bytes of one wavefront slot: two ping-pong buffers of three float4 arrays, and the hierarchy kernel's per-path results
@@ -1014,7 +1114,7 @@ extern "C" int pt_context_destroy(pt_context* c) {
   PT_FREE(c->d_rows); PT_FREE(c->d_meta); PT_FREE(c->d_normals); PT_FREE(c->d_mats); PT_FREE(c->d_lights); PT_FREE(c->d_state);
   PT_FREE(c->d_filt); PT_FREE(c->d_filt_ids); PT_FREE(c->d_bvh_nodes); PT_FREE(c->d_bvh_leaves); PT_FREE(c->d_bvh_meta);
   PT_FREE(c->d_ctrl); PT_FREE(c->d_live); PT_FREE(c->d_accum); PT_FREE(c->d_rgb); PT_FREE(c->d_rgba8);
-  PT_FREE(c->d_scratch); PT_FREE(c->d_light_k); PT_FREE(c->d_shadow);
+  PT_FREE(c->d_scratch); PT_FREE(c->d_light_k); PT_FREE(c->d_shadow); PT_FREE(c->d_ptab); PT_FREE(c->d_prim);
   PT_FREE(c->d_slab); PT_FREE(c->d_means); PT_FREE(c->d_base[0]); PT_FREE(c->d_base[1]);
 #undef PT_FREE
   for (int i = 0; i < pt_context::kSlots; i++) {
@@ -1297,6 +1397,7 @@ static int render_into(pt_context* c, uint32_t first_sample, uint32_t n_samples,
       P.div_band = make_fastdiv(band);
       P.q_offset = (uint32_t)c->geom_smem;
       P.cap = (uint32_t)cap;
+      P.ptab = c->ptab_on ? c->d_ptab : nullptr;
       const bool first = depth == 0, last = depth == max_depth - 1;
       cudaError_t e;
       if (first && last) e = launch_bounce<true, true>(c, 1, P, n_first, st);
@@ -1618,12 +1719,64 @@ extern "C" int pt_intersect(pt_context* c, int n, const float* origin, const flo
   return pt_intersect_ex(c, PT_HIT_FILTERED, n, origin, direction, geom_id, t, point, normal, nullptr);
 }
 
+extern "C" int pt_primary_hit(pt_context* c, uint64_t seed, int n, const uint32_t* pixel, const uint32_t* sample, int32_t* geom_id,
+                              float* t, float* point, float* normal, uint8_t* decided, uint64_t* fallbacks) {
+  CTX(c);
+  if (n < 0 || (n > 0 && (!pixel || !sample || !geom_id || !t || !point || !normal || !decided))) { pt_set_error_("bad arguments"); return PT_ERR_INVALID; }
+  if (c->mode != 0) { pt_set_error_("pt_primary_hit: the scene has %d geoms and uses the hierarchy, not the pair scan", c->n_geoms); return PT_ERR_STATE; }
+  if (fallbacks) *fallbacks = 0;
+  if (n == 0) return PT_OK;
+  for (int i = 0; i < n; i++)
+    if (pixel[i] >= c->npix) { pt_set_error_("pixel[%d] = %u outside the %u-pixel frame", i, pixel[i], c->npix); return PT_ERR_INVALID; }
+  const size_t v = 3 * (size_t)n;
+  Arena A(c);
+  if (int rc = A.reserve(2 * Arena::up(n * sizeof(uint32_t)) + 2 * Arena::up(v * sizeof(float)) + Arena::up(n * sizeof(float)) +
+                         Arena::up(n * sizeof(int)) + Arena::up(n) + 256)) return rc;
+  uint32_t *dp = A.take<uint32_t>(n), *ds = A.take<uint32_t>(n);
+  float *dt = A.take<float>(n), *dpnt = A.take<float>(v), *dn = A.take<float>(v);
+  int* did = A.take<int>(n);
+  uint8_t* ddec = A.take<uint8_t>(n);
+  unsigned long long* dfb = A.take<unsigned long long>(1);
+  CU(cudaMemcpyAsync(dp, pixel, n * sizeof(uint32_t), cudaMemcpyHostToDevice, c->stream));
+  CU(cudaMemcpyAsync(ds, sample, n * sizeof(uint32_t), cudaMemcpyHostToDevice, c->stream));
+  CU(cudaMemsetAsync(dfb, 0, sizeof(unsigned long long), c->stream));
+  k_primary_list<<<(n + kTile - 1) / kTile, kTile, c->geom_smem, c->stream>>>(c->cam, seed, c->g, c->n_geoms, c->filt, c->d_normals,
+                                                                               c->ptab_on ? c->d_ptab : nullptr, n, dp, ds, did, dt, dpnt, dn, ddec, dfb);
+  c->launches++;
+  CU(cudaGetLastError());
+  unsigned long long fb = 0;
+  CU(cudaMemcpyAsync(geom_id, did, n * sizeof(int), cudaMemcpyDeviceToHost, c->stream));
+  CU(cudaMemcpyAsync(t, dt, n * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+  CU(cudaMemcpyAsync(point, dpnt, v * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+  CU(cudaMemcpyAsync(normal, dn, v * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+  CU(cudaMemcpyAsync(decided, ddec, n, cudaMemcpyDeviceToHost, c->stream));
+  CU(cudaMemcpyAsync(&fb, dfb, sizeof(fb), cudaMemcpyDeviceToHost, c->stream));
+  CU(cudaStreamSynchronize(c->stream));
+  if (fallbacks) *fallbacks = fb;
+  return PT_OK;
+}
+
+extern "C" int pt_primary_table_info(pt_context* c, int* active, float* build_ms) {
+  CTX(c);
+  if (!active) { pt_set_error_("active is NULL"); return PT_ERR_INVALID; }
+  *active = c->ptab_on ? 1 : 0;
+  if (build_ms) {
+    // time one rebuild, host records to finished kernel: what a scene update or a filter-scale change pays for it
+    CU(cudaStreamSynchronize(c->stream));
+    const auto t0 = std::chrono::steady_clock::now();
+    if (int rc = build_primary_table(c)) return rc;
+    *build_ms = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t0).count();
+  }
+  return PT_OK;
+}
+
 extern "C" int pt_set_filter_scale(pt_context* c, float scale) {
   CTX(c);
   if (!(scale >= 0.0f) || !(scale <= 1e6f)) { pt_set_error_("filter scale %g outside [0, 1e6]", (double)scale); return PT_ERR_INVALID; }
   CU(cudaStreamSynchronize(c->stream));
   c->filter_scale = scale;
-  return upload_filter(c);
+  if (int rc = upload_filter(c)) return rc;
+  return build_primary_table(c);  // (its margin scales with the filter's)
 }
 
 extern "C" int pt_filter_stats(pt_context* c, uint64_t* fallbacks) {

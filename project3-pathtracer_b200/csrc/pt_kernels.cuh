@@ -129,7 +129,174 @@ struct BounceParams {
   uint32_t cap;                      // paths the in / out buffers hold (debug checks)
   uint32_t acc_s0, acc_stride;       // radiance of sample s goes to accum[(s - acc_s0) * acc_stride + pixel]: stride 0 = one image for
                                      // all samples (the rule), stride = pixels per frame = one image per sample (pt_stream_*)
+  const uint32_t* ptab;              // FIRST only: per-pixel candidate of the primary rays (k_primary_table), null = none
+                                     // (last member: the other kernels read the members before it at unchanged offsets)
 };
+
+// ---- the primary-ray table (DESIGN.md 3a "primary rays"): pinhole cameras, pair-scan scenes ----
+// Every primary ray of a pixel starts at the eye and points into the pixel's footprint, so the filter's answer is nearly
+// always the same for all of them.  k_primary_table works it out once per pixel, in binary64, for the footprint's
+// central ray against every filter shape grown by rho = D * (largest angle between a ray of the footprint and the
+// central ray): a grown shape the central ray enters at world distance s is entered by no ray of the footprint before
+// s.  Entry per pixel: (bits(lo2) & ~kKeyMask) | key of the candidate, kKeyMask = "no table decision".
+struct PrimRec {      // one filter shape at the eye, in the frame where it is a unit-free ball or box
+  double A[9];        // ray direction -> shape frame (identity for the world-space classes 0 and 2)
+  double ro[3];       // the eye in the shape frame
+  double h[3];        // ball: radius in h[0]; box: half extents
+  double g[3];        // growth of h per unit of world distance rho (ball: sigma_max(A) in g[0]; box: |row i of A|)
+  double D;           // no point of the shape is farther than D from the eye
+  double ew;          // world slack E_w of the filter at the eye
+  int ball, key;      // shape kind; 2 * pair + half of the filter scan
+};
+constexpr int kMaxPrimRecs = 128;
+// the pixel's footprint: d_c = unit central direction; returns the largest angle between d_c and the direction of any
+// primary ray raygen() makes for the pixel, rounding included, or a negative value when no bound is possible
+__device__ __forceinline__ double footprint_angle(const RaygenConsts& C, uint32_t pixel, double dc[3]) {
+  const double u = 5.9604644775390625e-8;  // 2^-24
+  const uint32_t yi = pixel / C.W;
+  const double x = (double)(pixel - yi * C.W), y = (double)yi, fw = C.fw, fh = C.fh;
+  // sx = 1 - 2 ((x + u0) / fw), u0 in [0, 1): the real interval, widened by the binary32 evaluation's error
+  const double ex = 16.0 * u * (1.0 + 2.0 * (x + 1.0) / fw), ey = 16.0 * u * (1.0 + 2.0 * (y + 1.0) / fh);
+  const double sx0 = 1.0 - 2.0 * (x + 1.0) / fw - ex, sx1 = 1.0 - 2.0 * x / fw + ex;
+  const double sy0 = 1.0 - 2.0 * (y + 1.0) / fh - ey, sy1 = 1.0 - 2.0 * y / fh + ey;
+  const double w[3] = {C.w.x, C.w.y, C.w.z}, H[3] = {C.Hh.x, C.Hh.y, C.Hh.z}, V[3] = {C.Vv.x, C.Vv.y, C.Vv.z};
+  // every v = w + H sx + V sy lies in one plane: |v| >= the plane's distance from the origin
+  double n[3] = {H[1] * V[2] - H[2] * V[1], H[2] * V[0] - H[0] * V[2], H[0] * V[1] - H[1] * V[0]};
+  const double nn = sqrt(n[0] * n[0] + n[1] * n[1] + n[2] * n[2]);
+  const double vmin = fabs(w[0] * n[0] + w[1] * n[1] + w[2] * n[2]) / nn;
+  const double nw = sqrt(w[0] * w[0] + w[1] * w[1] + w[2] * w[2]), nH = sqrt(H[0] * H[0] + H[1] * H[1] + H[2] * H[2]),
+               nV = sqrt(V[0] * V[0] + V[1] * V[1] + V[2] * V[2]);
+  // binary32 error of (w + H sx) + V sy, and of the normalisation, as an angle
+  const double ev = 8.0 * u * (nw + nH * fmax(fabs(sx0), fabs(sx1)) + nV * fmax(fabs(sy0), fabs(sy1)));
+  if (!(nn > 0) || !(vmin > 16.0 * ev)) return -1.0;
+  const double th_r = 2.0 * ev / vmin + 8.0 * u;
+  const double sxc = 0.5 * (sx0 + sx1), syc = 0.5 * (sy0 + sy1);
+  double l = 0.0;
+  for (int i = 0; i < 3; i++) { dc[i] = w[i] + H[i] * sxc + V[i] * syc; l += dc[i] * dc[i]; }
+  l = sqrt(l);
+  for (int i = 0; i < 3; i++) dc[i] /= l;
+  // the angle to d_c is quasi-convex over the rectangle (its sublevel sets are a plane cut through a convex cone), so
+  // its maximum is at a corner
+  double th = 0.0;
+  for (int k = 0; k < 4; k++) {
+    const double sx = (k & 1) ? sx1 : sx0, sy = (k & 2) ? sy1 : sy0;
+    double v[3];
+    for (int i = 0; i < 3; i++) v[i] = w[i] + H[i] * sx + V[i] * sy;
+    const double cx = v[1] * dc[2] - v[2] * dc[1], cy = v[2] * dc[0] - v[0] * dc[2], cz = v[0] * dc[1] - v[1] * dc[0];
+    th = fmax(th, atan2(sqrt(cx * cx + cy * cy + cz * cz), v[0] * dc[0] + v[1] * dc[1] + v[2] * dc[2]));
+  }
+  th = (th + th_r) * (1.0 + 1e-6) + 1e-12;
+  return th < 1.0 ? th : -1.0;  // (a cone of half-angle >= 1 rad: no table decision)
+}
+// smallest s >= 0 at which ro + s rw lies in the grown shape (rounded so that it is no later than the exact value),
+// +inf when it never does.  Both shapes are inflated by 1e-9 of their scale first, far above binary64 rounding.
+__device__ __forceinline__ double prim_entry(const PrimRec& R, const double rw[3], double rho) {
+  if (R.ball) {
+    const double r = R.h[0] + rho * R.g[0];
+    const double ro2 = R.ro[0] * R.ro[0] + R.ro[1] * R.ro[1] + R.ro[2] * R.ro[2];
+    const double a = rw[0] * rw[0] + rw[1] * rw[1] + rw[2] * rw[2];
+    const double b = R.ro[0] * rw[0] + R.ro[1] * rw[1] + R.ro[2] * rw[2];
+    const double c = ro2 - (r * r + 1e-9 * (ro2 + r * r));
+    const double disc = b * b - a * c;
+    if (disc < 0.0) return INFINITY;
+    const double sq = sqrt(disc);
+    if (-b + sq < 0.0) return INFINITY;  // behind the eye
+    return fmax((-b - sq) / a, 0.0);
+  }
+  double tn = 0.0, tf = INFINITY;
+  for (int i = 0; i < 3; i++) {
+    const double h = (R.h[i] + rho * R.g[i]) * (1.0 + 1e-9) + 1e-9 * fabs(R.ro[i]);
+    if (rw[i] == 0.0) {
+      if (fabs(R.ro[i]) > h) return INFINITY;
+      continue;
+    }
+    const double t1 = (-h - R.ro[i]) / rw[i], t2 = (h - R.ro[i]) / rw[i];
+    tn = fmax(tn, fmin(t1, t2));
+    tf = fmin(tf, fmax(t1, t2));
+  }
+  return tn <= tf ? tn : INFINITY;
+}
+__global__ void __launch_bounds__(128) k_primary_table(RaygenConsts C, const PrimRec* recs, int n_recs, double scale, uint32_t* tab) {
+  const uint32_t pixel = blockIdx.x * blockDim.x + threadIdx.x;
+  if (pixel >= C.npix) return;
+  double dc[3];
+  const double th = footprint_angle(C, pixel, dc);
+  uint32_t entry = kKeyMask;
+  if (th >= 0.0) {
+    double lo1 = INFINITY, lo2 = INFINITY;
+    int k1 = -1;
+    for (int j = 0; j < n_recs; j++) {
+      const PrimRec& R = recs[j];
+      double rw[3];
+      for (int i = 0; i < 3; i++) rw[i] = R.A[3 * i] * dc[0] + R.A[3 * i + 1] * dc[1] + R.A[3 * i + 2] * dc[2];
+      const double rho = scale * R.D * th * (1.0 + 1e-6);
+      const double s = prim_entry(R, rw, rho);
+      if (!(s < INFINITY)) continue;  // a proven miss for the whole footprint
+      const double lo = fmax(s - R.ew, 0.0);
+      if (lo < lo1) { lo2 = lo1; lo1 = lo; k1 = R.key; }
+      else lo2 = fmin(lo2, lo);
+    }
+    if (k1 >= 0 && lo2 > lo1) {
+      // lo2 rounded down to binary32 (a finite value: an entry's bits must not read as NaN), then its key bits cleared
+      float f = (float)fmin(lo2, 3.0e38);
+      if ((double)f > lo2) f = nextafterf(f, 0.0f);
+      entry = (__float_as_uint(f) & ~kKeyMask) | (uint32_t)k1;
+    }
+  }
+  tab[pixel] = entry;
+}
+
+// Closest hit of a primary ray, by a whole warp: the exact test of the table's candidate (`tab`, may be null) and, for
+// the lanes it does not settle, the filter scan and the exact test of its candidate -- ONE copy of the exact test for
+// both -- and, where that does not settle the ray either, the exact scan (return value: it ran).  The acceptance rule
+// is resolve_scan's, so the answer is the exact scan's, bit for bit.  `decided`: the table's candidate was confirmed.
+__device__ __forceinline__ bool primary_hit(const uint32_t* tab, const float4* fs, const FiltSoA& filt, const GeomSoA& g, int n_geoms,
+                                            bool valid, uint32_t pixel, f3 o, f3 d, Hit& h, bool& decided) {
+  ScanBest best;
+  best.k1 = -1; best.lo2 = 0.0f;
+  bool scan = valid, open = valid, from_tab = false, fell_back = false;
+  decided = false;
+  if (tab != nullptr && valid) {
+    const uint32_t e = __ldg(tab + pixel);
+    if ((e & kKeyMask) != kKeyMask) {
+      best.k1 = (int)(e & kKeyMask); best.lo2 = __uint_as_float(e & ~kKeyMask);
+      scan = false; from_tab = true;
+    }
+  }
+#pragma unroll 1
+  for (;;) {
+    if (__any_sync(0xffffffffu, scan)) {
+      if (scan) {
+        scan_init(best);
+        const ScanRay ray = make_scan_ray(o, d, filt.r_scene, filt.end[2] > filt.end[1]);
+        filter_scan(fs, 0, filt.end[3], filt.end, ray, best);
+      }
+    }
+    bool retry = false;
+    if (open && best.k1 >= 0) {
+      const int gi = __ldg(reinterpret_cast<const int*>(filt.ids) + best.k1);
+      const int type = best.k1 < 2 * filt.end[1] ? 0 : 1;
+      float dist;
+      f3 P;
+      int ncode;
+      DeferredGuard m;
+      const bool hit = exact_hit(type, __ldg(g.inv0 + gi), __ldg(g.inv1 + gi), __ldg(g.inv2 + gi), __ldg(g.fwd0 + gi),
+                                 __ldg(g.fwd1 + gi), __ldg(g.fwd2 + gi), o, d, dist, P, ncode, m);
+      if (!m.bad && hit && dist > 0 && dist < best.lo2) {
+        h.t = dist; h.id = gi; h.p = P; h.ncode = ncode;
+        decided = from_tab;
+      } else if (from_tab) {
+        retry = true;  // the footprint's candidate is not this ray's: the filter decides
+      } else {
+        closest_hit_exact(g, n_geoms, o, d, h);
+        fell_back = true;
+      }
+    }
+    if (!__any_sync(0xffffffffu, retry)) break;
+    scan = retry; open = retry; from_tab = false;
+  }
+  return fell_back;
+}
 
 // what changes from one depth of a wavefront to the next: the ping-pong buffers and the depth itself (a launch per depth
 // takes it from its parameters).  A single cooperative launch stepping through all depths of a small wavefront was
@@ -441,7 +608,11 @@ __device__ __forceinline__ void bounce_fused(const BounceParams& P, const DepthI
 
     Hit h;
     h.t = INFINITY; h.id = -1; h.p = mk(0, 0, 0); h.ncode = 0;
-    if (valid) {
+    if constexpr (FIRST) {  // primary rays: the per-pixel table first (pinhole cameras)
+      PT_CHECK(!valid || pixel < P.cam.npix);
+      bool decided;
+      if (primary_hit(P.ptab, fs, P.filt, P.g, P.n_geoms, valid, pixel, o, d, h, decided)) atomicAdd(&P.ctrl->fallbacks, 1u);
+    } else if (valid) {
       ScanBest best;
       scan_init(best);
       const ScanRay ray = make_scan_ray(o, d, P.filt.r_scene, P.filt.end[2] > P.filt.end[1]);
@@ -1141,6 +1312,36 @@ __global__ void __launch_bounds__(kTile) k_intersect_list(GeomSoA g, int n_geoms
   t[i] = h.id >= 0 ? h.t : -1.0f;
   p[3 * i] = h.p.x; p[3 * i + 1] = h.p.y; p[3 * i + 2] = h.p.z;
   nrm[3 * i] = nn.x; nrm[3 * i + 1] = nn.y; nrm[3 * i + 2] = nn.z;
+}
+
+// primary rays of (pixel, sample) pairs through depth 0's closest hit (primary_hit): table first, then the filter
+__global__ void __launch_bounds__(kTile) k_primary_list(RaygenConsts C, uint64_t seed, GeomSoA g, int n_geoms, FiltSoA filt,
+                                                        const float4* normals, const uint32_t* tab, int n, const uint32_t* pixel,
+                                                        const uint32_t* sample, int* id, float* t, float* p, float* nrm,
+                                                        uint8_t* decided, unsigned long long* fallbacks) {
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  const bool valid = i < n;
+  stage_filt(filt, 0, filt.end[3], reinterpret_cast<float4*>(smem_raw));
+  __syncthreads();
+  f3 oo = mk(0, 0, 0), dd = mk(0, 0, 1);
+  uint32_t px = 0;
+  if (valid) {
+    px = pixel[i];
+    PT_CHECK(px < C.npix);
+    raygen(C, seed, px, sample[i], oo, dd);
+  }
+  Hit h;
+  h.t = INFINITY; h.id = -1; h.p = mk(0, 0, 0); h.ncode = 0;
+  bool dec;
+  if (primary_hit(tab, reinterpret_cast<const float4*>(smem_raw), filt, g, n_geoms, valid, px, oo, dd, h, dec)) atomicAdd(fallbacks, 1ull);
+  if (!valid) return;
+  const f3 nn = h.id >= 0 ? hit_normal_table(normals, h) : mk(0, 0, 0);
+  id[i] = h.id;
+  t[i] = h.id >= 0 ? h.t : -1.0f;
+  p[3 * i] = h.p.x; p[3 * i + 1] = h.p.y; p[3 * i + 2] = h.p.z;
+  nrm[3 * i] = nn.x; nrm[3 * i + 1] = nn.y; nrm[3 * i + 2] = nn.z;
+  decided[i] = dec ? 1 : 0;
 }
 
 // ---- stream compaction on its own (README.md:63-70): stable, single pass, decoupled look-back ----

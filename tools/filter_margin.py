@@ -36,6 +36,24 @@ def main():
                     cells.append("%d/%.4f%%" % (bad, 100.0 * fb / len(gid)))
                 ctx.set_filter_scale(1.0)
                 print("%-22s %-14s %s" % (name, rname, "  ".join("%-9s" % c for c in cells)), flush=True)
+            # primary rays through depth 0's closest hit (per-pixel table first, then the filter): the table's margin
+            # scales with the filter's; cells = mismatches among all rays / share of rays the table decided
+            if ctx.primary_table_info()[0]:
+                spp = max(1, n // ctx.npix)
+                pixel = np.tile(np.arange(ctx.npix, dtype=np.uint32), spp)
+                sample = np.repeat(np.arange(spp, dtype=np.uint32), ctx.npix)
+                o, d = ctx.raygen(565, pixel, sample)
+                want = ctx.intersect(o, d, mode=pt.HIT_EXACT_SCAN)
+                cells = []
+                for s in scales:
+                    ctx.set_filter_scale(s)
+                    gid, t, p, nr, dec = ctx.primary_hit(565, pixel, sample)
+                    hit = want[0] >= 0
+                    bad = int(((gid != want[0]) | (t.view(np.uint32) != want[1].view(np.uint32))).sum()
+                              + (p[hit].view(np.uint32) != want[2][hit].view(np.uint32)).any(axis=1).sum())
+                    cells.append("%d/%.2f%%" % (bad, 100.0 * dec.mean()))
+                ctx.set_filter_scale(1.0)
+                print("%-22s %-14s %s" % (name, "primary", "  ".join("%-9s" % c for c in cells)), flush=True)
 
 
 if __name__ == "__main__":
