@@ -235,6 +235,14 @@ int pt_set_direct_lighting(pt_context* ctx, int on);
  * counts in full (no light sample at such an event).  Each scattering event is one segment of max_depth.  Media block
  * shadow rays like any refractive geom; nested or overlapping media are not modelled.  Drops an open sample stream. */
 int pt_set_subsurface(pt_context* ctx, int on);
+/* ---- glossy reflection (material.specularExponent, SPECEX in the scene format) ----
+ * Off by default: SPECEX is then carried but ignored, and every reflective material is a perfect mirror.  On: a sphere /
+ * cube whose material has REFL > 0, REFR <= 0, SPECEX > 0 and EMITTANCE <= 0 reflects into a Phong lobe of exponent SPECEX
+ * around the mirror direction (cos of the lobe angle distributed as c^(SPECEX+1)); a direction below the surface is
+ * folded back above it, so the lobe's albedo is exactly SPECRGB.  A glossy event is specular for direct light sampling:
+ * no light sample there, and the next emission its path meets counts in full.  Refractive materials keep ignoring
+ * SPECEX.  As SPECEX grows the lobe becomes the mirror.  Drops an open sample stream. */
+int pt_set_glossy(pt_context* ctx, int on);
 /* shadow rays traced by pt_render calls since the last pt_clear; n_lights (may be NULL) = emissive geoms of the scene */
 int pt_shadow_rays(pt_context* ctx, uint64_t* shadow_rays, int* n_lights);
 
@@ -260,6 +268,12 @@ int pt_calculate_transmission(int device, int n, const float* absorption, const 
  * scattered[i] = 0, direction[i] = 0 and weight[i] = calculateTransmission over distance[i]. */
 int pt_sample_medium(int device, int n, const float* absorption, const float* scatter, const float* distance, const float* u,
                      int32_t* scattered, float* s, float* direction, float* weight);
+/* the glossy lobe pt_set_glossy samples, for n reflections: outward normal[i] (x3) of the surface, incident[i] (x3) the
+ * unit direction of the arriving ray, exponent[i] = SPECEX > 0, u[i] = (u0, u1) in [0,1).  ns = normal[i] turned to face
+ * incident[i], r = reflect(ns, incident[i]); direction[i] = the sample of the lobe around r (unit length, dot with ns
+ * >= 0). */
+int pt_sample_glossy(int device, int n, const float* normal, const float* incident, const float* exponent, const float* u,
+                     float* direction);
 
 /* What the reference's own cudaRaytraceCore leaves in renderCam->image TODAY: its raytraceRay is a stub that overwrites
  * every pixel with generateRandomNumberFromThread(resolution, (float)iterations, x, y) (src/raytraceKernel.cu:29-36,

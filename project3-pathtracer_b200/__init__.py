@@ -198,6 +198,11 @@ class Context:
         (pt_set_subsurface); off by default"""
         _check(lib().pt_set_subsurface(self._h, C.c_int(1 if on else 0)))
 
+    def set_glossy(self, on=True):
+        """glossy reflection: reflective materials with SPECEX > 0 sample a Phong lobe around the mirror direction
+        (pt_set_glossy); off by default"""
+        _check(lib().pt_set_glossy(self._h, C.c_int(1 if on else 0)))
+
     def shadow_rays(self):
         """(shadow rays traced since the last clear, emissive geoms in the scene)"""
         n, nl = C.c_uint64(), C.c_int()
@@ -325,6 +330,19 @@ def sample_medium(absorption, scatter, distance, u, device=0):
     dirs, w = np.zeros((n, 3), np.float32), np.zeros((n, 3), np.float32)
     _check(lib().pt_sample_medium(C.c_int(device), C.c_int(n), _p(a), _p(sc), _p(d), _p(uu), _p(flag), _p(s), _p(dirs), _p(w)))
     return flag.astype(bool), s, dirs, w
+
+
+def sample_glossy(normal, incident, exponent, u, device=0):
+    """the glossy lobe of pt_set_glossy: outward normal (n, 3), incident direction (n, 3), SPECEX (n,) and uniforms
+    u = (n, 2) -> direction (n, 3), a Phong lobe of exponent SPECEX around the mirror direction of the normal turned to
+    face the incident ray, folded above the surface"""
+    nn, d = _arr(normal, np.float32).reshape(-1, 3), _arr(incident, np.float32).reshape(-1, 3)
+    e, uu = _arr(exponent, np.float32).ravel(), _arr(u, np.float32).reshape(-1, 2)
+    n = e.size
+    assert nn.shape[0] == n and d.shape[0] == n and uu.shape[0] == n
+    out = np.zeros((n, 3), np.float32)
+    _check(lib().pt_sample_glossy(C.c_int(device), C.c_int(n), _p(nn), _p(d), _p(e), _p(uu), _p(out)))
+    return out
 
 
 STUB_ORDER_DEVICE, STUB_ORDER_HOST = 0, 1

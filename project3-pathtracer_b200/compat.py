@@ -109,6 +109,10 @@ def set_subsurface(on):
     lib().pt_compat_set_subsurface(C.c_int(1 if on else 0))
 
 
+def set_glossy(on):
+    lib().pt_compat_set_glossy(C.c_int(1 if on else 0))
+
+
 def set_reference_stub(on):
     lib().pt_compat_set_reference_stub(C.c_int(1 if on else 0))
 

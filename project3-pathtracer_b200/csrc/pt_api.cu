@@ -19,6 +19,7 @@
 #include <atomic>
 #include <chrono>
 #include <thread>
+#include <type_traits>
 #include <functional>
 #include <vector>
 
@@ -65,6 +66,8 @@ struct FiltGeom {
   int key, cls, geom;  // key = 2 * pair + half, as the scan reports its candidate
   float c[3], k[6], wk[6], ew_c, ew_w;
 };
+// launch-time variants of a bounce kernel: index nee | medium << 1 | glossy << 2 (variant_index)
+constexpr int kVariants = 8;
 struct pt_context {
   int device = 0;
   int sm_count = 0;
@@ -83,6 +86,8 @@ struct pt_context {
   bool nee = false;            // pt_set_direct_lighting
   bool sss = false;            // pt_set_subsurface
   int n_media = 0;             // spheres / cubes whose material makes them a scattering medium (DESIGN.md 4)
+  bool glossy = false;         // pt_set_glossy
+  int n_glossy = 0;            // spheres / cubes whose material makes them glossy reflectors (DESIGN.md 4)
   float4* d_filt = nullptr;   // kFiltRows arrays of n_pairs float4: filter geometry (pt_filter.cuh)
   int2* d_filt_ids = nullptr;
   FiltSoA filt{};
@@ -127,11 +132,10 @@ struct pt_context {
   float4* d_accum = nullptr;
   float* d_rgb = nullptr;      // staging for packed RGB
   uchar4* d_rgba8 = nullptr;   // staging for the 8-bit resolve
-  int grid_blocks[4] = {0, 0, 0, 0};  // persistent grid per (FIRST,LAST) variant
-  int grid_blocks_nee[4] = {0, 0, 0, 0};  // ... of the direct-light-sampling variants
-  int grid_blocks_q[2] = {0, 0}, grid_blocks_q_nee[2] = {0, 0};  // k_bounce_q<LAST> (depths >= 1 of the linear mode)
-  int grid_blocks_med[4] = {0, 0, 0, 0}, grid_blocks_med_nee[4] = {0, 0, 0, 0};  // subsurface variants (not LAST: MediumOf)
-  int grid_blocks_q_med = 0, grid_blocks_q_med_nee = 0;                          // ... of k_bounce_q<false>
+  // persistent grid per (FIRST,LAST) slot and launch-time variant (variant_index); 0 = no such variant (NeeOf, MediumOf,
+  // GlossyOf)
+  int grid_blocks[4][kVariants] = {};
+  int grid_blocks_q[2][kVariants] = {};  // k_bounce_q<LAST> (depths >= 1 of the linear mode)
   size_t q_smem_total = 0;            // k_bounce_q: filter geometry + the warps' candidate queues
   int q_mode = 0;                     // depths >= 1, few geoms: 0 = per depth by the scene's measured survival (h_policy),
                                       // 1 = always k_bounce_q, 2 = always the fused k_bounce (PT_B200_FUSED=1 / =0 force 2 / 1)
@@ -699,6 +703,26 @@ struct NeeOf { static constexpr bool value = !(F && L); };
 // are those of the plain kernel
 template <bool L>
 struct MediumOf { static constexpr bool value = !L; };
+// the glossy-reflection variant of LAST: none, for the same reason -- the last segment stores no direction, so the
+// direction a glossy event samples there is never used
+template <bool L>
+struct GlossyOf { static constexpr bool value = !L; };
+
+static int variant_index(bool nee, bool med, bool gl) { return (nee ? 1 : 0) | (med ? 2 : 0) | (gl ? 4 : 0); }
+// Calls fn(N, M, G) with the launch-time switches (nee, med, gl) of a bounce kernel of segment kind (F, L) as
+// std::bool_constant arguments: one instantiation per combination.  A switch the kind has no variant for (NeeOf,
+// MediumOf, GlossyOf) is passed as false, so no instantiation is made that cannot be launched.
+template <bool F, bool L, typename Fn>
+static auto with_variant(bool nee, bool med, bool gl, Fn&& fn) {
+  auto g = [&](auto N, auto M) { return gl ? fn(N, M, std::bool_constant<GlossyOf<L>::value>{}) : fn(N, M, std::false_type{}); };
+  auto m = [&](auto N) { return med ? g(N, std::bool_constant<MediumOf<L>::value>{}) : g(N, std::false_type{}); };
+  return nee ? m(std::bool_constant<NeeOf<F, L>::value>{}) : m(std::false_type{});
+}
+// a variant index whose switches segment kind (F, L) has a variant for
+template <bool F, bool L>
+static bool has_variant(int v) {
+  return ((v & 1) == 0 || NeeOf<F, L>::value) && ((v & 2) == 0 || MediumOf<L>::value) && ((v & 4) == 0 || GlossyOf<L>::value);
+}
 
 // resident CTAs per SM of one bounce kernel with `smem` bytes of dynamic shared memory
 template <typename K>
@@ -711,58 +735,38 @@ static int fit_kernel(K kernel, int threads, size_t smem, bool carveout, int* pe
 
 template <bool F, bool L>
 static int setup_variant(pt_context* c, int slot) {
-  int per_sm = 0, per_sm_nee = 0, per_sm_med = 1, per_sm_med_nee = 1;
-  constexpr bool N = NeeOf<F, L>::value, M = MediumOf<L>::value;
-  int rc;
-  if (c->mode) {  // (many geoms: one kernel for every depth, primary rays come from k_raygen_wf)
-    CU(cudaFuncSetAttribute(k_bounce_bvh<L>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kBvhSmemBytes));
-    CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_bounce_bvh<L>, kBvhThreads, kBvhSmemBytes));
-    CU(cudaFuncSetAttribute(k_bounce_bvh<L, N>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kBvhSmemBytes));
-    CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm_nee, k_bounce_bvh<L, N>, kBvhThreads, kBvhSmemBytes));
-    if constexpr (M) {
-      if ((rc = fit_kernel(k_bounce_bvh<L, false, true>, kBvhThreads, kBvhSmemBytes, false, &per_sm_med))) return rc;
-      if ((rc = fit_kernel(k_bounce_bvh<L, N, true>, kBvhThreads, kBvhSmemBytes, false, &per_sm_med_nee))) return rc;
-    }
-  } else {
-    CU(cudaFuncSetAttribute(k_bounce<F, L>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c->smem_bytes));
-    CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_bounce<F, L>, kBounceThreads, c->smem_bytes));
-    CU(cudaFuncSetAttribute(k_bounce<F, L, N>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c->smem_bytes));
-    CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm_nee, k_bounce<F, L, N>, kBounceThreads, c->smem_bytes));
-    if constexpr (M) {
-      if ((rc = fit_kernel(k_bounce<F, L, false, true>, kBounceThreads, c->smem_bytes, false, &per_sm_med))) return rc;
-      if ((rc = fit_kernel(k_bounce<F, L, N, true>, kBounceThreads, c->smem_bytes, false, &per_sm_med_nee))) return rc;
-    }
+  for (int v = 0; v < kVariants; v++) {
+    c->grid_blocks[slot][v] = 0;
+    if (!has_variant<F, L>(v)) continue;
+    int per_sm = 0;
+    // (many geoms: one kernel for every depth, primary rays come from k_raygen_wf)
+    const int rc = with_variant<F, L>(v & 1, v & 2, v & 4, [&](auto N, auto M, auto G) {
+      constexpr bool n = decltype(N)::value, m = decltype(M)::value, g = decltype(G)::value;
+      return c->mode ? fit_kernel(k_bounce_bvh<L, n, m, g>, kBvhThreads, kBvhSmemBytes, false, &per_sm)
+                     : fit_kernel(k_bounce<F, L, n, m, g>, kBounceThreads, c->smem_bytes, false, &per_sm);
+    });
+    if (rc) return rc;
+    if (per_sm < 1) { pt_set_error_("k_bounce does not fit on an SM"); return PT_ERR_CUDA; }
+    c->grid_blocks[slot][v] = per_sm * c->sm_count;
   }
-  if (per_sm < 1 || per_sm_nee < 1 || per_sm_med < 1 || per_sm_med_nee < 1) { pt_set_error_("k_bounce does not fit on an SM"); return PT_ERR_CUDA; }
-  c->grid_blocks[slot] = per_sm * c->sm_count;
-  c->grid_blocks_nee[slot] = per_sm_nee * c->sm_count;
-  c->grid_blocks_med[slot] = M ? per_sm_med * c->sm_count : 0;
-  c->grid_blocks_med_nee[slot] = M ? per_sm_med_nee * c->sm_count : 0;
   return PT_OK;
 }
 
+// (the last segment never samples a light, but it honours the no-emission flag: k_bounce_q<true> has NEE variants --
+// NeeOf<false, L>)
 template <bool L>
 static int setup_variant_q(pt_context* c, int slot) {
-  int per_sm = 0, per_sm_nee = 0, per_sm_med = 1, per_sm_med_nee = 1;
-  constexpr bool N = true;  // (the last segment never samples a light, but it honours the no-emission flag)
-  constexpr bool M = MediumOf<L>::value;
-  int rc;
-  CU(cudaFuncSetAttribute(k_bounce_q<L>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c->q_smem_total));
-  CU(cudaFuncSetAttribute(k_bounce_q<L>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-  CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_bounce_q<L>, kQThreads, c->q_smem_total));
-  CU(cudaFuncSetAttribute(k_bounce_q<L, N>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c->q_smem_total));
-  CU(cudaFuncSetAttribute(k_bounce_q<L, N>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-  CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm_nee, k_bounce_q<L, N>, kQThreads, c->q_smem_total));
-  if constexpr (M) {
-    if ((rc = fit_kernel(k_bounce_q<L, false, true>, kQThreads, c->q_smem_total, true, &per_sm_med))) return rc;
-    if ((rc = fit_kernel(k_bounce_q<L, N, true>, kQThreads, c->q_smem_total, true, &per_sm_med_nee))) return rc;
-  }
-  if (per_sm < 1 || per_sm_nee < 1 || per_sm_med < 1 || per_sm_med_nee < 1) { pt_set_error_("k_bounce_q does not fit on an SM"); return PT_ERR_CUDA; }
-  c->grid_blocks_q[slot] = per_sm * c->sm_count;
-  c->grid_blocks_q_nee[slot] = per_sm_nee * c->sm_count;
-  if (M) {
-    c->grid_blocks_q_med = per_sm_med * c->sm_count;
-    c->grid_blocks_q_med_nee = per_sm_med_nee * c->sm_count;
+  for (int v = 0; v < kVariants; v++) {
+    c->grid_blocks_q[slot][v] = 0;
+    if (!has_variant<false, L>(v)) continue;
+    int per_sm = 0;
+    const int rc = with_variant<false, L>(v & 1, v & 2, v & 4, [&](auto N, auto M, auto G) {
+      return fit_kernel(k_bounce_q<L, decltype(N)::value, decltype(M)::value, decltype(G)::value>, kQThreads, c->q_smem_total,
+                        true, &per_sm);
+    });
+    if (rc) return rc;
+    if (per_sm < 1) { pt_set_error_("k_bounce_q does not fit on an SM"); return PT_ERR_CUDA; }
+    c->grid_blocks_q[slot][v] = per_sm * c->sm_count;
   }
   return PT_OK;
 }
@@ -1003,10 +1007,12 @@ static int upload_scene(pt_context* c, const pt_static_geom* geoms, int n_geoms,
   CU(cudaMemcpyAsync(c->d_meta, meta.data(), meta.size() * sizeof(int2), cudaMemcpyHostToDevice, c->stream));
   CU(cudaMemcpyAsync(c->d_mats, mats, (size_t)n_mats * sizeof(pt_material), cudaMemcpyHostToDevice, c->stream));
   c->n_media = 0;
+  c->n_glossy = 0;
   for (int i = 0; i < n_geoms; i++) {
     if (geoms[i].type > 1) continue;
     const pt_material& mm = mats[geoms[i].materialid];
     if (mm.hasRefractive > 0 && mm.hasScatter > 0 && mm.reducedScatterCoefficient > 0) c->n_media++;
+    if (!(mm.emittance > 0) && !(mm.hasRefractive > 0) && mm.hasReflective > 0 && mm.specularExponent > 0) c->n_glossy++;
   }
   std::vector<float> geom_k;
   const std::vector<float4> lights = build_lights(geoms, n_geoms, mats, &geom_k);
@@ -1240,22 +1246,20 @@ extern "C" int pt_clear(pt_context* c) {
 template <bool F, bool L>
 static cudaError_t launch_bounce(pt_context* c, int slot, const BounceParams& P, uint32_t n_upper, cudaStream_t st) {
   const bool nee = c->nee && c->n_lights > 0 && NeeOf<F, L>::value;
-  constexpr bool N = NeeOf<F, L>::value, M = MediumOf<L>::value;
-  const bool med = M && c->sss && c->n_media > 0;  // (no medium in the scene: the plain kernels, same results)
-  uint32_t grid = (uint32_t)(med ? (nee ? c->grid_blocks_med_nee[slot] : c->grid_blocks_med[slot])
-                                 : (nee ? c->grid_blocks_nee[slot] : c->grid_blocks[slot]));
+  const bool med = MediumOf<L>::value && c->sss && c->n_media > 0;  // (no medium in the scene: the plain kernels, same results)
+  const bool gl = GlossyOf<L>::value && c->glossy && c->n_glossy > 0;  // (likewise without a glossy geom)
+  const int v = variant_index(nee, med, gl);
+  uint32_t grid = (uint32_t)c->grid_blocks[slot][v];
   // depths >= 1, few geoms: second half re-batched by winner type -- unless the scene keeps nearly all its paths alive
   // at this depth (closed rooms), where the fused kernel is faster; unknown yet (first wavefronts of a scene): re-batched
   const bool use_q = c->q_mode == 1 || (c->q_mode == 0 && ((volatile int*)c->h_policy)[P.depth] != 2);
   if (!F && !c->mode && use_q) {
-    uint32_t gq = (uint32_t)(med ? (nee ? c->grid_blocks_q_med_nee : c->grid_blocks_q_med)
-                                 : (nee ? c->grid_blocks_q_nee[L ? 1 : 0] : c->grid_blocks_q[L ? 1 : 0]));
+    uint32_t gq = (uint32_t)c->grid_blocks_q[L ? 1 : 0][v];
     const uint32_t ctas = (n_upper + kQThreads - 1) / kQThreads;  // one unit per warp at least
     if (ctas < gq) gq = ctas ? ctas : 1;
-    if (med && nee) k_bounce_q<L, N, M><<<gq, kQThreads, c->q_smem_total, st>>>(P);
-    else if (med) k_bounce_q<L, false, M><<<gq, kQThreads, c->q_smem_total, st>>>(P);
-    else if (nee) k_bounce_q<L, N><<<gq, kQThreads, c->q_smem_total, st>>>(P);
-    else k_bounce_q<L><<<gq, kQThreads, c->q_smem_total, st>>>(P);
+    with_variant<F, L>(nee, med, gl, [&](auto N, auto M, auto G) {
+      k_bounce_q<L, decltype(N)::value, decltype(M)::value, decltype(G)::value><<<gq, kQThreads, c->q_smem_total, st>>>(P);
+    });
   } else if (c->mode) {
     if (F) {  // primary rays into the wavefront's input buffers
       const uint32_t blocks = (n_upper + 255u) / 256u, most = (uint32_t)c->sm_count * 8u;
@@ -1264,17 +1268,15 @@ static cudaError_t launch_bounce(pt_context* c, int slot, const BounceParams& P,
     }
     const uint32_t ctas = (n_upper + kPoolMin * (kBvhThreads / 32) - 1) / (kPoolMin * (kBvhThreads / 32));  // a (smallest) pool per warp at least
     if (ctas < grid) grid = ctas ? ctas : 1;
-    if (med && nee) k_bounce_bvh<L, N, M><<<grid, kBvhThreads, kBvhSmemBytes, st>>>(P);
-    else if (med) k_bounce_bvh<L, false, M><<<grid, kBvhThreads, kBvhSmemBytes, st>>>(P);
-    else if (nee) k_bounce_bvh<L, N><<<grid, kBvhThreads, kBvhSmemBytes, st>>>(P);
-    else k_bounce_bvh<L><<<grid, kBvhThreads, kBvhSmemBytes, st>>>(P);
+    with_variant<F, L>(nee, med, gl, [&](auto N, auto M, auto G) {
+      k_bounce_bvh<L, decltype(N)::value, decltype(M)::value, decltype(G)::value><<<grid, kBvhThreads, kBvhSmemBytes, st>>>(P);
+    });
   } else {
     const uint32_t ctas = (n_upper + kBounceThreads - 1) / kBounceThreads;  // one unit per warp at least
     if (ctas < grid) grid = ctas ? ctas : 1;
-    if (med && nee) k_bounce<F, L, N, M><<<grid, kBounceThreads, c->smem_bytes, st>>>(P);
-    else if (med) k_bounce<F, L, false, M><<<grid, kBounceThreads, c->smem_bytes, st>>>(P);
-    else if (nee) k_bounce<F, L, N><<<grid, kBounceThreads, c->smem_bytes, st>>>(P);
-    else k_bounce<F, L><<<grid, kBounceThreads, c->smem_bytes, st>>>(P);
+    with_variant<F, L>(nee, med, gl, [&](auto N, auto M, auto G) {
+      k_bounce<F, L, decltype(N)::value, decltype(M)::value, decltype(G)::value><<<grid, kBounceThreads, c->smem_bytes, st>>>(P);
+    });
   }
   c->launches++;
   return cudaGetLastError();
@@ -1813,6 +1815,13 @@ extern "C" int pt_set_subsurface(pt_context* c, int on) {
   c->sss = on != 0;
   return PT_OK;
 }
+extern "C" int pt_set_glossy(pt_context* c, int on) {
+  CTX(c);
+  if (int rc = stream_discard(c)) return rc;
+  CU(cudaStreamSynchronize(c->stream));
+  c->glossy = on != 0;
+  return PT_OK;
+}
 extern "C" int pt_shadow_rays(pt_context* c, uint64_t* shadow_rays, int* n_lights) {
   CTX(c);
   if (!shadow_rays) { pt_set_error_("shadow_rays is NULL"); return PT_ERR_INVALID; }
@@ -2007,6 +2016,29 @@ extern "C" int pt_sample_medium(int device, int n, const float* absorption, cons
   CU(cudaMemcpy(s, ds, n * sizeof(float), cudaMemcpyDeviceToHost));
   CU(cudaMemcpy(direction, ddir, n3 * sizeof(float), cudaMemcpyDeviceToHost));
   CU(cudaMemcpy(weight, dw, n3 * sizeof(float), cudaMemcpyDeviceToHost));
+  return PT_OK;
+}
+
+extern "C" int pt_sample_glossy(int device, int n, const float* normal, const float* incident, const float* exponent,
+                                const float* u, float* direction) {
+  if (n < 0 || (n > 0 && (!normal || !incident || !exponent || !u || !direction))) {
+    pt_set_error_("bad arguments");
+    return PT_ERR_INVALID;
+  }
+  if (n == 0) return PT_OK;
+  if (int rc = select_device_(device)) return rc;
+  const size_t n3 = 3 * (size_t)n;
+  // one arena: normal, incident, exponent, u in; direction out
+  DevBuf<float> buf;
+  CU(buf.alloc(n3 + n3 + n + 2 * (size_t)n + n3));
+  float *dn = buf.p, *di = dn + n3, *de = di + n3, *du = de + n, *ddir = du + 2 * (size_t)n;
+  CU(cudaMemcpy(dn, normal, n3 * sizeof(float), cudaMemcpyHostToDevice));
+  CU(cudaMemcpy(di, incident, n3 * sizeof(float), cudaMemcpyHostToDevice));
+  CU(cudaMemcpy(de, exponent, n * sizeof(float), cudaMemcpyHostToDevice));
+  CU(cudaMemcpy(du, u, 2 * (size_t)n * sizeof(float), cudaMemcpyHostToDevice));
+  k_sample_glossy<<<(n + 255) / 256, 256>>>(n, dn, di, de, du, ddir);
+  CU(cudaGetLastError());
+  CU(cudaMemcpy(direction, ddir, n3 * sizeof(float), cudaMemcpyDeviceToHost));
   return PT_OK;
 }
 

@@ -1,21 +1,22 @@
 // pt_kernels.cuh -- the wavefront kernels (sm_100a).
 //
-//   k_bounce<FIRST,LAST,NEE,MEDIUM>  one path segment for every live path of the wavefront, fused (few geoms: depth 0, and every depth
+//   k_bounce<FIRST,LAST,NEE,MEDIUM,GLOSSY>  one path segment for every live path of the wavefront, fused (few geoms: depth 0, and every depth
 //                           of scenes that keep nearly all their paths alive):
 //                           [FIRST: raygen + depth of field]  (raycastFromCameraKernel, src/raytraceKernel.cu:40-45)
 //                           closest hit over SoA geometry staged in shared memory (src/intersections.h:74-117)
 //                           BSDF sampling with Philox (calculateBSDF, src/interactions.h:99-104), absorption inside glass
 //                           (calculateTransmission, :31-33), [NEE: direct light sampling, src/intersections.h:133-182]
 //                           [MEDIUM: subsurface scattering inside media, calculateScatterAndAbsorption, :36-39]
+//                           [GLOSSY: glossy reflection, a Phong lobe around the mirror direction (SPECEX)]
 //                           radiance accumulation in HBM (the running image of src/raytraceKernel.cu:118-120,154)
 //                           stream compaction of the survivors (README.md:63-70): warp ballot -> ranks inside a 32-path
 //                           unit, one slot-reserving atomic per unit, survivors written once to the other ping-pong
 //                           buffer.
 //                         Persistent CTAs; warps take units from a ticket counter and never wait for each other; the
 //                         live count never visits the host.
-//   k_bounce_q<LAST,NEE,MEDIUM>  depths >= 1 of few-geom scenes: the same segment with its second half (exact test of the filter's
+//   k_bounce_q<LAST,NEE,MEDIUM,GLOSSY>  depths >= 1 of few-geom scenes: the same segment with its second half (exact test of the filter's
 //                         candidate, shading, compaction) re-batched by winner type in per-warp shared-memory queues
-//   k_raygen_wf + k_bounce_bvh<LAST,NEE,MEDIUM>   scenes with many geoms: primary rays into the wavefront's buffers, then one kernel
+//   k_raygen_wf + k_bounce_bvh<LAST,NEE,MEDIUM,GLOSSY>   scenes with many geoms: primary rays into the wavefront's buffers, then one kernel
 //                         for every depth -- pooled traversal of the hierarchy (pt_bvh.cuh) with lane refill, exact
 //                         tests and shading unit by unit
 //   k_shadow_lin / k_shadow_bvh   direct light sampling: the shadow rays a depth queued, traced by a launch of their own
@@ -462,7 +463,8 @@ __device__ PT_NEE_INLINE void direct_light(const BounceParams& P, const DepthIO&
 // shared memory (`fs`; few geoms) or walk the hierarchy (many geoms).  NEE: direct light sampling at diffuse bounces; `cos_b` > 0 = the path's
 // previous event was one (the cosine of the direction it sampled travels in throughput.w): a light it reaches by itself is
 // weighted by the balance heuristic against that event's light sample.  MEDIUM: subsurface scattering (shade() may return 4,
-// a scattering event inside a medium geom: the path goes on, without a light sample).
+// a scattering event inside a medium geom: the path goes on, without a light sample).  GLOSSY: glossy reflection (a glossy
+// event is kind 1, like a mirror: no light sample, and its path carries cos_b = 0).
 // Deferred output (k_bounce_q): a batch's survivors wait in shared memory while the atomic that reserves their slots is
 // in flight, and are written one batch later -- the warp never waits for the atomic (it was 7 % of the stall samples:
 // one address per depth takes 0.6 atomics per nanosecond, and their latency under that load exceeds a whole shading pass).
@@ -487,7 +489,7 @@ __device__ __forceinline__ void deferred_flush(DeferredOut& W, const BounceParam
   __syncwarp();  // the staging rows may be overwritten now
 }
 
-template <bool LAST, bool TABLE, bool NEE, bool DEFER = false, bool LINEAR = TABLE, bool MEDIUM = false>
+template <bool LAST, bool TABLE, bool NEE, bool DEFER = false, bool LINEAR = TABLE, bool MEDIUM = false, bool GLOSSY = false>
 __device__ __forceinline__ void shade_and_compact(const BounceParams& P, const DepthIO& io, const float4* fs, uint32_t lane, bool hit, const Hit& h, f3 o, f3 d, f3 thr,
                                                   uint32_t pixel, uint32_t sample, float cos_b, DeferredOut* W = nullptr) {
   // a path survives this segment unless it left the scene or reached a light; the slot of the unit's survivors
@@ -524,7 +526,7 @@ __device__ __forceinline__ void shade_and_compact(const BounceParams& P, const D
     if (NEE && !LAST) ns = dot(d, n) < 0 ? n : neg(n);  // the shading normal shade() uses
     const float4* frame = nullptr;
     if (TABLE && h.ncode != 8) frame = P.normals + (size_t)gi * kNormalRows + kFrameRow0 + 4 * ((h.ncode & 3) + ((h.ncode & 4) ? 3 : 0));
-    const int kind = shade<MEDIUM>(m, P.g, gi, h.p, n, frame, P.keys, pixel, sample, io.depth, o, d, thr, L);
+    const int kind = shade<MEDIUM, GLOSSY>(m, P.g, gi, h.p, n, frame, P.keys, pixel, sample, io.depth, o, d, thr, L);
     if (kind == 3) {
       // a light reached by a direction the diffuse bounce before sampled itself: balance heuristic against that bounce's
       // light sample (cos_b = cosine of this direction at the bounce, 0 = camera ray / specular event: full weight)
@@ -569,7 +571,7 @@ __device__ __forceinline__ void shade_and_compact(const BounceParams& P, const D
 
 // Few geoms (every BASELINE config but the 10k one): linear scan over the filter pairs staged in shared memory.
 // The body of one depth, by every warp of a persistent grid (`fs` = the staged filter pairs):
-template <bool FIRST, bool LAST, bool NEE, bool MEDIUM>
+template <bool FIRST, bool LAST, bool NEE, bool MEDIUM, bool GLOSSY>
 __device__ __forceinline__ void bounce_fused(const BounceParams& P, const DepthIO& io, const float4* fs, uint32_t lane) {
   const uint32_t n_in = FIRST ? P.n_first : P.ctrl->count[io.depth];
   if (FIRST && blockIdx.x == 0 && threadIdx.x == 0) P.ctrl->count[0] = n_in;
@@ -620,18 +622,18 @@ __device__ __forceinline__ void bounce_fused(const BounceParams& P, const DepthI
       if (resolve_scan(best, P.filt, P.g, P.n_geoms, o, d, h)) atomicAdd(&P.ctrl->fallbacks, 1u);
     }
 
-    shade_and_compact<LAST, true, NEE, false, true, MEDIUM>(P, io, fs, lane, valid && h.id >= 0, h, o, d, thr, pixel, sample, cos_b);
+    shade_and_compact<LAST, true, NEE, false, true, MEDIUM, GLOSSY>(P, io, fs, lane, valid && h.id >= 0, h, o, d, thr, pixel, sample, cos_b);
     }
   }
 }
 
-template <bool FIRST, bool LAST, bool NEE = false, bool MEDIUM = false>
+template <bool FIRST, bool LAST, bool NEE = false, bool MEDIUM = false, bool GLOSSY = false>
 __global__ void __launch_bounds__(kBounceThreads, PT_MIN_BLOCKS) k_bounce(const __grid_constant__ BounceParams P) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   // ---- filter geometry: staged once per CTA ----
   stage_filt(P.filt, 0, P.filt.end[3], reinterpret_cast<float4*>(smem_raw));
   __syncthreads();  // the only CTA-wide barrier
-  bounce_fused<FIRST, LAST, NEE, MEDIUM>(P, depth_io(P), reinterpret_cast<const float4*>(smem_raw), threadIdx.x & 31u);
+  bounce_fused<FIRST, LAST, NEE, MEDIUM, GLOSSY>(P, depth_io(P), reinterpret_cast<const float4*>(smem_raw), threadIdx.x & 31u);
 }
 
 // ---- k_bounce_q: the same segment with the second half RE-BATCHED BY WINNER TYPE (depths >= 1, few geoms) ----
@@ -690,7 +692,7 @@ __device__ __forceinline__ void cp_async16(void* smem, const void* gmem) {
 __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
 __device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_group 0;" ::: "memory"); }
 
-template <bool LAST, bool NEE = false, bool MEDIUM = false>
+template <bool LAST, bool NEE = false, bool MEDIUM = false, bool GLOSSY = false>
 __global__ void __launch_bounds__(kQThreads, PT_Q_MIN_BLOCKS) k_bounce_q(const __grid_constant__ BounceParams P) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   const uint32_t lane = threadIdx.x & 31u;
@@ -772,9 +774,9 @@ __global__ void __launch_bounds__(kQThreads, PT_Q_MIN_BLOCKS) k_bounce_q(const _
       const float cos_b = NEE ? c.w : 0.0f;
       __syncwarp();  // the popped entries are in registers: the next push may overwrite them
 #if PT_Q_DEFER_OUT
-      shade_and_compact<LAST, true, NEE, true, true, MEDIUM>(P, io, fs, lane, valid && h.id >= 0, h, o, d, thr, pixel, sample, cos_b, &W);
+      shade_and_compact<LAST, true, NEE, true, true, MEDIUM, GLOSSY>(P, io, fs, lane, valid && h.id >= 0, h, o, d, thr, pixel, sample, cos_b, &W);
 #else
-      shade_and_compact<LAST, true, NEE, false, true, MEDIUM>(P, io, fs, lane, valid && h.id >= 0, h, o, d, thr, pixel, sample, cos_b);
+      shade_and_compact<LAST, true, NEE, false, true, MEDIUM, GLOSSY>(P, io, fs, lane, valid && h.id >= 0, h, o, d, thr, pixel, sample, cos_b);
 #endif
     }
     if (!more) break;
@@ -901,17 +903,17 @@ __device__ __forceinline__ void load_path(const BounceParams& P, uint32_t idx, f
 #ifndef PT_BVH_TABLE
 #define PT_BVH_TABLE 0  // normals, tangent frames and the material row from the per-geom table, as in the few-geom kernels
 #endif
-template <bool LAST, bool NEE, bool MEDIUM>
+template <bool LAST, bool NEE, bool MEDIUM, bool GLOSSY>
 __device__ __noinline__ void shade_unit_bvh(const BounceParams& P, const DepthIO& io, uint32_t lane, bool hit, const Hit& h, f3 o, f3 d,
                                             f3 thr, uint32_t pixel, uint32_t sample, float cos_b) {
-  shade_and_compact<LAST, PT_BVH_TABLE != 0, NEE, false, false, MEDIUM>(P, io, nullptr, lane, hit, h, o, d, thr, pixel, sample, cos_b);
+  shade_and_compact<LAST, PT_BVH_TABLE != 0, NEE, false, false, MEDIUM, GLOSSY>(P, io, nullptr, lane, hit, h, o, d, thr, pixel, sample, cos_b);
 }
 
 // `n` (<= 32, warp-uniform) deferred paths, taken from the top of the warp's list: paths whose two nearest candidates
 // did not settle the closest hit (a third geom is in the way: ~0.1 % of the segments) go through the EXACT traversal --
 // every candidate leaf along the ray that can still matter is tested exactly -- all lanes together, then shading and
 // compaction as a unit of their own.
-template <bool LAST, bool NEE, bool MEDIUM>
+template <bool LAST, bool NEE, bool MEDIUM, bool GLOSSY>
 __device__ __noinline__ void run_deferred(const BounceParams& P, const uint32_t* list, uint32_t n) {
   const uint32_t lane = threadIdx.x & 31u;
   const DepthIO io = depth_io(P);
@@ -928,7 +930,7 @@ __device__ __noinline__ void run_deferred(const BounceParams& P, const uint32_t*
     bvh_exact(P.bvh, P.g, o, d, P.filt.r_scene, h);
   }
   if (lane == 0) atomicAdd(&P.ctrl->fallbacks, n);  // statistics: segments that needed the exact traversal
-  shade_unit_bvh<LAST, NEE, MEDIUM>(P, io, lane, valid && h.id >= 0, h, o, d, thr, pixel, sample, cos_b);
+  shade_unit_bvh<LAST, NEE, MEDIUM, GLOSSY>(P, io, lane, valid && h.id >= 0, h, o, d, thr, pixel, sample, cos_b);
 }
 
 // the next pool of a warp: kPool paths while plenty are left, fewer (down to kPoolMin) when the wavefront runs out, so
@@ -1062,7 +1064,7 @@ __device__ __forceinline__ bool bvh_resolve2(const BounceParams& P, uint32_t lan
 
 // phase 2 of a pool: exact test of the candidates, shading, compaction, unit by unit; paths that two candidates do not
 // settle go to the warp's list for the exact traversal, which is run whenever the list holds a unit's worth
-template <bool LAST, bool NEE, bool MEDIUM>
+template <bool LAST, bool NEE, bool MEDIUM, bool GLOSSY>
 __device__ __forceinline__ void bvh_phase2(const BounceParams& P, const DepthIO& io, BvhWarpSmem& S, uint32_t lane, uint32_t base, uint32_t n_pool,
                                            uint32_t& n_defer) {
 #pragma unroll 1
@@ -1085,11 +1087,11 @@ __device__ __forceinline__ void bvh_phase2(const BounceParams& P, const DepthIO&
     PT_CHECK(n_defer + __popc(dmask) <= (uint32_t)kDeferCap);
     if (defer) S.defer[n_defer + __popc(dmask & ((1u << lane) - 1u))] = base + j;
     n_defer += __popc(dmask);
-    shade_unit_bvh<LAST, NEE, MEDIUM>(P, io, lane, valid && !defer && h.id >= 0, h, o, d, thr, pixel, sample, cos_b);
+    shade_unit_bvh<LAST, NEE, MEDIUM, GLOSSY>(P, io, lane, valid && !defer && h.id >= 0, h, o, d, thr, pixel, sample, cos_b);
     if (n_defer >= kUnit) {
       __syncwarp();
       n_defer -= kUnit;
-      run_deferred<LAST, NEE, MEDIUM>(P, S.defer + n_defer, kUnit);
+      run_deferred<LAST, NEE, MEDIUM, GLOSSY>(P, S.defer + n_defer, kUnit);
       __syncwarp();
     }
   }
@@ -1098,7 +1100,7 @@ __device__ __forceinline__ void bvh_phase2(const BounceParams& P, const DepthIO&
 // (Traversal and exact test + shading as two kernels were measured: the traversal loop alone fits 48 registers only with
 // spills, and at 64 it takes as long as this kernel takes for both phases -- in one kernel the arithmetic of the warps in
 // phase 2 fills the issue slots that the warps in phase 1 leave while they wait for nodes: 2.51 vs 3.00 Gseg/s.)
-template <bool LAST, bool NEE = false, bool MEDIUM = false>
+template <bool LAST, bool NEE = false, bool MEDIUM = false, bool GLOSSY = false>
 __global__ void __launch_bounds__(kBvhThreads, PT_BVH_MIN_BLOCKS) k_bounce_bvh(const __grid_constant__ BounceParams P) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   const uint32_t lane = threadIdx.x & 31u;
@@ -1111,11 +1113,11 @@ __global__ void __launch_bounds__(kBvhThreads, PT_BVH_MIN_BLOCKS) k_bounce_bvh(c
   while (bvh_take_pool(&P.ctrl->tile_ctr[P.depth], n_in, n_warps, lane, base, n_pool)) {
     bvh_phase1(P, S, lane, n_in, base, n_pool);
     __syncwarp();  // (the pool's results were written by this warp: ordered for its other lanes)
-    bvh_phase2<LAST, NEE, MEDIUM>(P, io, S, lane, base, n_pool, n_defer);
+    bvh_phase2<LAST, NEE, MEDIUM, GLOSSY>(P, io, S, lane, base, n_pool, n_defer);
   }
   if (n_defer) {
     __syncwarp();
-    run_deferred<LAST, NEE, MEDIUM>(P, S.defer, n_defer);
+    run_deferred<LAST, NEE, MEDIUM, GLOSSY>(P, S.defer, n_defer);
   }
 }
 

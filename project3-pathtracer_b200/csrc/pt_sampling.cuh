@@ -153,5 +153,17 @@ __global__ void k_sample_medium(int n, const float* absorption, const float* sca
   dir[3 * i] = e.dir.x; dir[3 * i + 1] = e.dir.y; dir[3 * i + 2] = e.dir.z;
   weight[3 * i] = e.weight.x; weight[3 * i + 1] = e.weight.y; weight[3 * i + 2] = e.weight.z;
 }
+// u = (u0, u1) per entry: the two uniforms the renderer takes from the segment's Philox block (u[0], u[1]); the shading
+// normal faces the incident direction as in shade()
+__global__ void k_sample_glossy(int n, const float* normal, const float* incident, const float* exponent, const float* u,
+                                float* dir) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const f3 nn = mk(normal[3 * i], normal[3 * i + 1], normal[3 * i + 2]);
+  const f3 d = mk(incident[3 * i], incident[3 * i + 1], incident[3 * i + 2]);
+  const f3 ns = dot(d, nn) < 0 ? nn : neg(nn);
+  const f3 g = sample_glossy(ns, d, exponent[i], u[2 * i], u[2 * i + 1]);
+  dir[3 * i] = g.x; dir[3 * i + 1] = g.y; dir[3 * i + 2] = g.z;
+}
 
 }  // namespace ptd

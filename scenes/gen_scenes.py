@@ -14,6 +14,9 @@
                          cube of the sample scene's material 5 coefficients (REFRIOR 2.2, ABSCOEFF .02 5.1 5.7,
                          RSCTCOEFF 13) with SCATTER 1 -- and RGB 1 1 1, since the sample's RGB 0 0 0 would stop every
                          path that refracts into them
+  cornell_glossy.txt     glossy reflection (pt_set_glossy / pt_render glossy=1): the closed room of cornell_sss.txt with
+                         three glossy spheres (SPECEX 10, 100, 1000), a glossy back wall (SPECEX 30) and a perfect
+                         mirror sphere (SPECEX 0) for contrast
   procedural(n, seed)    config 3: n spheres/cubes, i.i.d. type, centre, scale, rotation (radians) and material from a
                          fixed seed; written on demand (python scenes/gen_scenes.py --procedural 10000 out.txt)
 """
@@ -145,6 +148,37 @@ def cornell_sss():
     return scene_text(mats, cam, objs)
 
 
+def cornell_glossy():
+    mats = [
+        ((.85, .85, .85), 0, (1, 1, 1), 0, 0, 0, 0, (0, 0, 0), 0, 0),        # 0 white
+        ((.63, .06, .04), 0, (1, 1, 1), 0, 0, 0, 0, (0, 0, 0), 0, 0),        # 1 red
+        ((.15, .48, .09), 0, (1, 1, 1), 0, 0, 0, 0, (0, 0, 0), 0, 0),        # 2 green
+        ((1, 1, 1), 0, (0, 0, 0), 0, 0, 0, 0, (0, 0, 0), 0, 15),             # 3 light
+        ((1, 1, 1), 10, (.95, .8, .5), 1, 0, 0, 0, (0, 0, 0), 0, 0),         # 4 glossy, SPECEX 10
+        ((1, 1, 1), 100, (.9, .9, .9), 1, 0, 0, 0, (0, 0, 0), 0, 0),         # 5 glossy, SPECEX 100
+        ((1, 1, 1), 1000, (.6, .75, .95), 1, 0, 0, 0, (0, 0, 0), 0, 0),      # 6 glossy, SPECEX 1000
+        ((1, 1, 1), 0, (.95, .95, .95), 1, 0, 0, 0, (0, 0, 0), 0, 0),        # 7 perfect mirror
+        ((1, 1, 1), 30, (.8, .8, .8), 1, 0, 0, 0, (0, 0, 0), 0, 0),          # 8 glossy wall, SPECEX 30
+    ]
+    z0 = (0, 0, 0)
+    objs = [
+        ("cube", 0, [((0, 0, 0), z0, (10, .01, 10))]),      # floor
+        ("cube", 0, [((0, 10, 0), z0, (10, .01, 10))]),     # ceiling
+        ("cube", 8, [((0, 5, -5), z0, (10, 10, .01))]),     # back: glossy
+        ("cube", 0, [((0, 5, 5), z0, (10, 10, .01))]),      # front (behind the camera): closed room
+        ("cube", 1, [((-5, 5, 0), z0, (.01, 10, 10))]),     # left
+        ("cube", 2, [((5, 5, 0), z0, (.01, 10, 10))]),      # right
+        ("cube", 3, [((0, 9.9, 0), z0, (3, .15, 3))]),      # emissive panel
+        ("sphere", 4, [((-3, 1, -1.5), z0, (2, 2, 2))]),
+        ("sphere", 5, [((-1, 1, -1.5), z0, (2, 2, 2))]),
+        ("sphere", 6, [((1, 1, -1.5), z0, (2, 2, 2))]),
+        ("sphere", 7, [((3, 1, -1.5), z0, (2, 2, 2))]),     # mirror
+    ]
+    cam = dict(res=(800, 800), fovy=30, iterations=1024, file="cornell_glossy.png",
+               frames=[((0, 5, 4.8), (0, -0.25, -1), (0, 1, 0))])
+    return scene_text(mats, cam, objs)
+
+
 def sample_animated(n_frames=3, res=(800, 800), iterations=5000):
     """the sample scene with a bouncing sphere, a sliding camera and one per-frame array for every object
     (the reference's loader reads `frame k` blocks into per-frame arrays, src/scene.cpp:82-128, and its main loop
@@ -184,7 +218,8 @@ def procedural(n, seed=565, res=(1920, 1080), iterations=1024):
 
 def write_all():
     files = {"sample.txt": sample_scene(), "cornell_glass_dof.txt": cornell_glass_dof(),
-             "sample_4k.txt": sample_scene((3840, 2160), 16384), "cornell_sss.txt": cornell_sss()}
+             "sample_4k.txt": sample_scene((3840, 2160), 16384), "cornell_sss.txt": cornell_sss(),
+             "cornell_glossy.txt": cornell_glossy()}
     for name, text in files.items():
         with open(os.path.join(HERE, name), "w") as f:
             f.write(text)
