@@ -243,6 +243,14 @@ int pt_set_subsurface(pt_context* ctx, int on);
  * no light sample there, and the next emission its path meets counts in full.  Refractive materials keep ignoring
  * SPECEX.  As SPECEX grows the lobe becomes the mirror.  Drops an open sample stream. */
 int pt_set_glossy(pt_context* ctx, int on);
+/* ---- Russian roulette ----
+ * first_depth 0 (the default): off, a path ends only when it leaves the scene, reaches a light or runs out of max_depth
+ * segments.  first_depth k in [1, 63]: at every depth d with k <= d < max_depth - 1 whose closest hit is not emissive, a
+ * path with throughput thr goes on with probability q = max(thr.x, thr.y, thr.z) rounded up to a multiple of 2^-24 (1 for
+ * max >= 1: no draw, thr unchanged) and is reweighted to thr / q; otherwise it ends there, without shading or light
+ * sample.  The estimator stays unbiased; paths whose throughput never falls below 1 are never touched.  The draw is u[0]
+ * of Philox block 129 + d.  Other values return PT_ERR_INVALID.  Drops an open sample stream. */
+int pt_set_russian_roulette(pt_context* ctx, int first_depth);
 /* shadow rays traced by pt_render calls since the last pt_clear; n_lights (may be NULL) = emissive geoms of the scene */
 int pt_shadow_rays(pt_context* ctx, uint64_t* shadow_rays, int* n_lights);
 

@@ -94,6 +94,8 @@ int pt_compat_set_ahead(int samples);
 int pt_compat_set_direct_lighting(int on); /* pt_set_direct_lighting for the calls that follow (default off) */
 int pt_compat_set_subsurface(int on);      /* pt_set_subsurface for the calls that follow (default off) */
 int pt_compat_set_glossy(int on);          /* pt_set_glossy for the calls that follow (default off) */
+int pt_compat_set_russian_roulette(int first_depth); /* pt_set_russian_roulette for the calls that follow (default 0: off);
+                                                      * PT_ERR_INVALID outside [0, 63] */
 /* 1: cudaRaytraceCore behaves exactly like the UNMODIFIED reference does today -- its raytraceRay is a stub that fills
  * renderCam->image with per-pixel noise and converts that to the PBO (src/raytraceKernel.cu:93-104,149-154) -- so a
  * build can be checked against the reference before the renderer is switched on (default 0) */

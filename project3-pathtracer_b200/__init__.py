@@ -203,6 +203,12 @@ class Context:
         (pt_set_glossy); off by default"""
         _check(lib().pt_set_glossy(self._h, C.c_int(1 if on else 0)))
 
+    def set_russian_roulette(self, first_depth):
+        """Russian roulette from depth `first_depth` (1..63; 0 = off, the default): a path whose throughput has fallen
+        below 1 ends at random and the survivors are reweighted, an unbiased way to stop spending segments on paths that
+        contribute little (pt_set_russian_roulette)"""
+        _check(lib().pt_set_russian_roulette(self._h, C.c_int(int(first_depth))))
+
     def shadow_rays(self):
         """(shadow rays traced since the last clear, emissive geoms in the scene)"""
         n, nl = C.c_uint64(), C.c_int()

@@ -113,6 +113,11 @@ def set_glossy(on):
     lib().pt_compat_set_glossy(C.c_int(1 if on else 0))
 
 
+def set_russian_roulette(first_depth):
+    if lib().pt_compat_set_russian_roulette(C.c_int(int(first_depth))) != 0:
+        raise ValueError("Russian roulette takes 0 (off) or a first depth in [1, 63], not %r" % (first_depth,))
+
+
 def set_reference_stub(on):
     lib().pt_compat_set_reference_stub(C.c_int(1 if on else 0))
 

@@ -34,11 +34,12 @@ struct Cache {
   const camera* last_cam = nullptr;
   int last_frame = -1, last_iter = 0;
   bool streaming = false;  // a sample stream is open on ctx: samples last_iter, last_iter + 1, ... are traced ahead
-  int stream_depth = 0, stream_direct = 0, stream_sss = 0, stream_glossy = 0;
+  int stream_depth = 0, stream_direct = 0, stream_sss = 0, stream_glossy = 0, stream_rr = 0;
   unsigned long long stream_seed = 0;
   int direct_applied = -1; // pt_set_direct_lighting drops the stream: only called when the value changes
   int sss_applied = -1;    // ... and so does pt_set_subsurface
   int glossy_applied = -1; // ... and pt_set_glossy
+  int rr_applied = -1;     // ... and pt_set_russian_roulette
   std::vector<float> scaled;
   void* pinned = nullptr;  // renderCam->image, page-locked in place while a sequence of calls keeps arriving for it
   size_t pinned_bytes = 0;
@@ -53,6 +54,7 @@ int g_ahead = 8;   // samples per group traced ahead of the calls (pt_compat_set
 int g_direct = 0;  // pt_compat_set_direct_lighting
 int g_sss = 0;     // pt_compat_set_subsurface
 int g_glossy = 0;  // pt_compat_set_glossy
+int g_rr = 0;      // pt_compat_set_russian_roulette
 int g_stub = 0;    // pt_compat_set_reference_stub
 int g_status = PT_OK;
 
@@ -88,6 +90,11 @@ extern "C" int pt_compat_set_ahead(int samples) {
 extern "C" int pt_compat_set_direct_lighting(int on) { g_direct = on != 0; return PT_OK; }
 extern "C" int pt_compat_set_subsurface(int on) { g_sss = on != 0; return PT_OK; }
 extern "C" int pt_compat_set_glossy(int on) { g_glossy = on != 0; return PT_OK; }
+extern "C" int pt_compat_set_russian_roulette(int first_depth) {
+  if (first_depth < 0 || first_depth > 63) return PT_ERR_INVALID;
+  g_rr = first_depth;
+  return PT_OK;
+}
 extern "C" int pt_compat_set_reference_stub(int on) { g_stub = on != 0; return PT_OK; }
 extern "C" int pt_compat_last_status(void) { return g_status; }
 // The caller reads renderCam->image after every call (src/main.cpp:118-131), so its D2H copy cannot go away; but a
@@ -184,7 +191,8 @@ void cudaRaytraceCore(uchar4* PBOpos, camera* renderCam, int frame, int iteratio
   const bool in_sequence = !scene_changed && g.last_cam == renderCam && g.last_frame == frame && iterations == g.last_iter + 1;
   // the stream of samples traced ahead goes on if this call is the next iteration with the same settings
   const bool stream_ok = g.streaming && in_sequence && g.stream_depth == g_depth && g.stream_seed == g_seed &&
-                         g.stream_direct == g_direct && g.stream_sss == g_sss && g.stream_glossy == g_glossy;
+                         g.stream_direct == g_direct && g.stream_sss == g_sss && g.stream_glossy == g_glossy &&
+                         g.stream_rr == g_rr;
   if (!stream_ok) {
     if (g.streaming) { g.streaming = false; if ((rc = pt_stream_end(g.ctx))) return fail(rc); }
     if (iterations == 1) {
@@ -209,9 +217,13 @@ void cudaRaytraceCore(uchar4* PBOpos, camera* renderCam, int frame, int iteratio
       if ((rc = pt_set_glossy(g.ctx, g_glossy))) return fail(rc);
       g.glossy_applied = g_glossy;
     }
+    if (g.rr_applied != g_rr) {
+      if ((rc = pt_set_russian_roulette(g.ctx, g_rr))) return fail(rc);
+      g.rr_applied = g_rr;
+    }
     if ((rc = pt_stream_begin(g.ctx, (uint32_t)(iterations - 1), (uint32_t)(iterations - 1), g_depth, g_seed, (uint32_t)g_ahead))) return fail(rc);
     g.streaming = true; g.stream_depth = g_depth; g.stream_seed = g_seed; g.stream_direct = g_direct; g.stream_sss = g_sss;
-    g.stream_glossy = g_glossy;
+    g.stream_glossy = g_glossy; g.stream_rr = g_rr;
   }
   if (in_sequence || iterations == 1) pin(renderCam->image, npix * 3 * sizeof(float), iterations == 1);  // a render loop, not a one-off call
   if ((rc = pt_stream_next(g.ctx, reinterpret_cast<float*>(renderCam->image), PBOpos, nullptr))) return fail(rc);

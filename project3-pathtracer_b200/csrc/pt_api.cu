@@ -66,8 +66,8 @@ struct FiltGeom {
   int key, cls, geom;  // key = 2 * pair + half, as the scan reports its candidate
   float c[3], k[6], wk[6], ew_c, ew_w;
 };
-// launch-time variants of a bounce kernel: index nee | medium << 1 | glossy << 2 (variant_index)
-constexpr int kVariants = 8;
+// launch-time variants of a bounce kernel: index nee | medium << 1 | glossy << 2 | roulette << 3 (variant_index)
+constexpr int kVariants = 16;
 struct pt_context {
   int device = 0;
   int sm_count = 0;
@@ -88,6 +88,7 @@ struct pt_context {
   int n_media = 0;             // spheres / cubes whose material makes them a scattering medium (DESIGN.md 4)
   bool glossy = false;         // pt_set_glossy
   int n_glossy = 0;            // spheres / cubes whose material makes them glossy reflectors (DESIGN.md 4)
+  int rr_first = 0;            // pt_set_russian_roulette: first roulette depth, 0 = off
   float4* d_filt = nullptr;   // kFiltRows arrays of n_pairs float4: filter geometry (pt_filter.cuh)
   int2* d_filt_ids = nullptr;
   FiltSoA filt{};
@@ -133,7 +134,7 @@ struct pt_context {
   float* d_rgb = nullptr;      // staging for packed RGB
   uchar4* d_rgba8 = nullptr;   // staging for the 8-bit resolve
   // persistent grid per (FIRST,LAST) slot and launch-time variant (variant_index); 0 = no such variant (NeeOf, MediumOf,
-  // GlossyOf)
+  // GlossyOf, RouletteOf)
   int grid_blocks[4][kVariants] = {};
   int grid_blocks_q[2][kVariants] = {};  // k_bounce_q<LAST> (depths >= 1 of the linear mode)
   size_t q_smem_total = 0;            // k_bounce_q: filter geometry + the warps' candidate queues
@@ -707,21 +708,31 @@ struct MediumOf { static constexpr bool value = !L; };
 // direction a glossy event samples there is never used
 template <bool L>
 struct GlossyOf { static constexpr bool value = !L; };
+// the Russian-roulette variant of (FIRST, LAST): none for the first segment, whose throughput is 1, nor for the last one,
+// which continues nowhere -- roulette runs at neither (DESIGN.md 4)
+template <bool F, bool L>
+struct RouletteOf { static constexpr bool value = !F && !L; };
 
-static int variant_index(bool nee, bool med, bool gl) { return (nee ? 1 : 0) | (med ? 2 : 0) | (gl ? 4 : 0); }
-// Calls fn(N, M, G) with the launch-time switches (nee, med, gl) of a bounce kernel of segment kind (F, L) as
+static int variant_index(bool nee, bool med, bool gl, bool rr) {
+  return (nee ? 1 : 0) | (med ? 2 : 0) | (gl ? 4 : 0) | (rr ? 8 : 0);
+}
+// Calls fn(N, M, G, R) with the launch-time switches (nee, med, gl, rr) of a bounce kernel of segment kind (F, L) as
 // std::bool_constant arguments: one instantiation per combination.  A switch the kind has no variant for (NeeOf,
-// MediumOf, GlossyOf) is passed as false, so no instantiation is made that cannot be launched.
+// MediumOf, GlossyOf, RouletteOf) is passed as false, so no instantiation is made that cannot be launched.
 template <bool F, bool L, typename Fn>
-static auto with_variant(bool nee, bool med, bool gl, Fn&& fn) {
-  auto g = [&](auto N, auto M) { return gl ? fn(N, M, std::bool_constant<GlossyOf<L>::value>{}) : fn(N, M, std::false_type{}); };
+static auto with_variant(bool nee, bool med, bool gl, bool rr, Fn&& fn) {
+  auto r = [&](auto N, auto M, auto G) {
+    return rr ? fn(N, M, G, std::bool_constant<RouletteOf<F, L>::value>{}) : fn(N, M, G, std::false_type{});
+  };
+  auto g = [&](auto N, auto M) { return gl ? r(N, M, std::bool_constant<GlossyOf<L>::value>{}) : r(N, M, std::false_type{}); };
   auto m = [&](auto N) { return med ? g(N, std::bool_constant<MediumOf<L>::value>{}) : g(N, std::false_type{}); };
   return nee ? m(std::bool_constant<NeeOf<F, L>::value>{}) : m(std::false_type{});
 }
 // a variant index whose switches segment kind (F, L) has a variant for
 template <bool F, bool L>
 static bool has_variant(int v) {
-  return ((v & 1) == 0 || NeeOf<F, L>::value) && ((v & 2) == 0 || MediumOf<L>::value) && ((v & 4) == 0 || GlossyOf<L>::value);
+  return ((v & 1) == 0 || NeeOf<F, L>::value) && ((v & 2) == 0 || MediumOf<L>::value) && ((v & 4) == 0 || GlossyOf<L>::value) &&
+         ((v & 8) == 0 || RouletteOf<F, L>::value);
 }
 
 // resident CTAs per SM of one bounce kernel with `smem` bytes of dynamic shared memory
@@ -740,10 +751,10 @@ static int setup_variant(pt_context* c, int slot) {
     if (!has_variant<F, L>(v)) continue;
     int per_sm = 0;
     // (many geoms: one kernel for every depth, primary rays come from k_raygen_wf)
-    const int rc = with_variant<F, L>(v & 1, v & 2, v & 4, [&](auto N, auto M, auto G) {
-      constexpr bool n = decltype(N)::value, m = decltype(M)::value, g = decltype(G)::value;
-      return c->mode ? fit_kernel(k_bounce_bvh<L, n, m, g>, kBvhThreads, kBvhSmemBytes, false, &per_sm)
-                     : fit_kernel(k_bounce<F, L, n, m, g>, kBounceThreads, c->smem_bytes, false, &per_sm);
+    const int rc = with_variant<F, L>(v & 1, v & 2, v & 4, v & 8, [&](auto N, auto M, auto G, auto R) {
+      constexpr bool n = decltype(N)::value, m = decltype(M)::value, g = decltype(G)::value, r = decltype(R)::value;
+      return c->mode ? fit_kernel(k_bounce_bvh<L, n, m, g, r>, kBvhThreads, kBvhSmemBytes, false, &per_sm)
+                     : fit_kernel(k_bounce<F, L, n, m, g, r>, kBounceThreads, c->smem_bytes, false, &per_sm);
     });
     if (rc) return rc;
     if (per_sm < 1) { pt_set_error_("k_bounce does not fit on an SM"); return PT_ERR_CUDA; }
@@ -760,9 +771,9 @@ static int setup_variant_q(pt_context* c, int slot) {
     c->grid_blocks_q[slot][v] = 0;
     if (!has_variant<false, L>(v)) continue;
     int per_sm = 0;
-    const int rc = with_variant<false, L>(v & 1, v & 2, v & 4, [&](auto N, auto M, auto G) {
-      return fit_kernel(k_bounce_q<L, decltype(N)::value, decltype(M)::value, decltype(G)::value>, kQThreads, c->q_smem_total,
-                        true, &per_sm);
+    const int rc = with_variant<false, L>(v & 1, v & 2, v & 4, v & 8, [&](auto N, auto M, auto G, auto R) {
+      return fit_kernel(k_bounce_q<L, decltype(N)::value, decltype(M)::value, decltype(G)::value, decltype(R)::value>, kQThreads,
+                        c->q_smem_total, true, &per_sm);
     });
     if (rc) return rc;
     if (per_sm < 1) { pt_set_error_("k_bounce_q does not fit on an SM"); return PT_ERR_CUDA; }
@@ -1248,7 +1259,8 @@ static cudaError_t launch_bounce(pt_context* c, int slot, const BounceParams& P,
   const bool nee = c->nee && c->n_lights > 0 && NeeOf<F, L>::value;
   const bool med = MediumOf<L>::value && c->sss && c->n_media > 0;  // (no medium in the scene: the plain kernels, same results)
   const bool gl = GlossyOf<L>::value && c->glossy && c->n_glossy > 0;  // (likewise without a glossy geom)
-  const int v = variant_index(nee, med, gl);
+  const bool rr = RouletteOf<F, L>::value && c->rr_first > 0 && P.depth >= (uint32_t)c->rr_first;  // (a roulette depth)
+  const int v = variant_index(nee, med, gl, rr);
   uint32_t grid = (uint32_t)c->grid_blocks[slot][v];
   // depths >= 1, few geoms: second half re-batched by winner type -- unless the scene keeps nearly all its paths alive
   // at this depth (closed rooms), where the fused kernel is faster; unknown yet (first wavefronts of a scene): re-batched
@@ -1257,8 +1269,9 @@ static cudaError_t launch_bounce(pt_context* c, int slot, const BounceParams& P,
     uint32_t gq = (uint32_t)c->grid_blocks_q[L ? 1 : 0][v];
     const uint32_t ctas = (n_upper + kQThreads - 1) / kQThreads;  // one unit per warp at least
     if (ctas < gq) gq = ctas ? ctas : 1;
-    with_variant<F, L>(nee, med, gl, [&](auto N, auto M, auto G) {
-      k_bounce_q<L, decltype(N)::value, decltype(M)::value, decltype(G)::value><<<gq, kQThreads, c->q_smem_total, st>>>(P);
+    with_variant<F, L>(nee, med, gl, rr, [&](auto N, auto M, auto G, auto R) {
+      k_bounce_q<L, decltype(N)::value, decltype(M)::value, decltype(G)::value, decltype(R)::value>
+          <<<gq, kQThreads, c->q_smem_total, st>>>(P);
     });
   } else if (c->mode) {
     if (F) {  // primary rays into the wavefront's input buffers
@@ -1268,14 +1281,16 @@ static cudaError_t launch_bounce(pt_context* c, int slot, const BounceParams& P,
     }
     const uint32_t ctas = (n_upper + kPoolMin * (kBvhThreads / 32) - 1) / (kPoolMin * (kBvhThreads / 32));  // a (smallest) pool per warp at least
     if (ctas < grid) grid = ctas ? ctas : 1;
-    with_variant<F, L>(nee, med, gl, [&](auto N, auto M, auto G) {
-      k_bounce_bvh<L, decltype(N)::value, decltype(M)::value, decltype(G)::value><<<grid, kBvhThreads, kBvhSmemBytes, st>>>(P);
+    with_variant<F, L>(nee, med, gl, rr, [&](auto N, auto M, auto G, auto R) {
+      k_bounce_bvh<L, decltype(N)::value, decltype(M)::value, decltype(G)::value, decltype(R)::value>
+          <<<grid, kBvhThreads, kBvhSmemBytes, st>>>(P);
     });
   } else {
     const uint32_t ctas = (n_upper + kBounceThreads - 1) / kBounceThreads;  // one unit per warp at least
     if (ctas < grid) grid = ctas ? ctas : 1;
-    with_variant<F, L>(nee, med, gl, [&](auto N, auto M, auto G) {
-      k_bounce<F, L, decltype(N)::value, decltype(M)::value, decltype(G)::value><<<grid, kBounceThreads, c->smem_bytes, st>>>(P);
+    with_variant<F, L>(nee, med, gl, rr, [&](auto N, auto M, auto G, auto R) {
+      k_bounce<F, L, decltype(N)::value, decltype(M)::value, decltype(G)::value, decltype(R)::value>
+          <<<grid, kBounceThreads, c->smem_bytes, st>>>(P);
     });
   }
   c->launches++;
@@ -1820,6 +1835,17 @@ extern "C" int pt_set_glossy(pt_context* c, int on) {
   if (int rc = stream_discard(c)) return rc;
   CU(cudaStreamSynchronize(c->stream));
   c->glossy = on != 0;
+  return PT_OK;
+}
+extern "C" int pt_set_russian_roulette(pt_context* c, int first_depth) {
+  CTX(c);
+  if (first_depth < 0 || first_depth > kMaxDepth - 1) {
+    pt_set_error_("first_depth %d: Russian roulette takes 0 (off) or a first depth in [1, %d]", first_depth, kMaxDepth - 1);
+    return PT_ERR_INVALID;
+  }
+  if (int rc = stream_discard(c)) return rc;
+  CU(cudaStreamSynchronize(c->stream));
+  c->rr_first = first_depth;
   return PT_OK;
 }
 extern "C" int pt_shadow_rays(pt_context* c, uint64_t* shadow_rays, int* n_lights) {

@@ -6,11 +6,12 @@
 // cudaRaytraceCore call per sample, keeps the image in HBM, and writes PNG (out= / bmp=1 to override).
 //
 //   pt_render scene=<file> [frame=<n>] [spp=<n>] [depth=<n>] [seed=<n>] [gpus=<n>] [out=<name>] [bmp=1]
-//             [rotat=degrees] [wavefront=<paths>] [json=1] [direct=1] [sss=1] [glossy=1]
+//             [rotat=degrees] [wavefront=<paths>] [json=1] [direct=1] [sss=1] [glossy=1] [rr=<k>]
 //
 // direct=1 turns on direct light sampling at diffuse bounces (pt_set_direct_lighting); sss=1 turns on subsurface
 // scattering inside refractive geoms whose material has SCATTER and RSCTCOEFF (pt_set_subsurface); glossy=1 turns on
-// glossy reflection for reflective materials with SPECEX > 0 (pt_set_glossy).
+// glossy reflection for reflective materials with SPECEX > 0 (pt_set_glossy); rr=K turns on Russian roulette from depth K
+// (pt_set_russian_roulette, 1 <= K <= 63).
 //
 // gpus=N shards the samples of each frame over N GPUs by contiguous sample-index blocks (one host thread and one
 // context per GPU) and combines the accumulation buffers with one NCCL reduce.
@@ -31,7 +32,7 @@ static int die(const char* what) {
 
 int main(int argc, char** argv) {
   std::string scene_path, out_name;
-  int frame = -1, spp = -1, depth = 8, gpus = 1, bmp = 0, rot_deg = 0, json = 0, direct = 0, sss = 0, glossy = 0;
+  int frame = -1, spp = -1, depth = 8, gpus = 1, bmp = 0, rot_deg = 0, json = 0, direct = 0, sss = 0, glossy = 0, rr = 0;
   unsigned long long seed = 0, wavefront = 0;
   for (int i = 1; i < argc; i++) {
     std::string tok = argv[i];
@@ -52,11 +53,12 @@ int main(int argc, char** argv) {
     else if (k == "direct") direct = atoi(v.c_str());
     else if (k == "sss") sss = atoi(v.c_str());
     else if (k == "glossy") glossy = atoi(v.c_str());
+    else if (k == "rr") rr = atoi(v.c_str());
   }
   if (scene_path.empty()) {
     // main.cpp:38-41
     fprintf(stderr, "Error: scene file needed!\nusage: pt_render scene=<file> [frame=<n>] [spp=<n>] [depth=<n>] [seed=<n>] "
-                    "[gpus=<n>] [out=<name>] [bmp=1] [rotat=degrees] [wavefront=<paths>] [json=1] [direct=1] [sss=1] [glossy=1]\n");
+                    "[gpus=<n>] [out=<name>] [bmp=1] [rotat=degrees] [wavefront=<paths>] [json=1] [direct=1] [sss=1] [glossy=1] [rr=<k>]\n");
     return 1;
   }
   pt_scene* sc = nullptr;
@@ -87,6 +89,7 @@ int main(int argc, char** argv) {
       if (pt_set_direct_lighting(ctx[g], direct)) return die("direct");
       if (pt_set_subsurface(ctx[g], sss)) return die("sss");
       if (pt_set_glossy(ctx[g], glossy)) return die("glossy");
+      if (pt_set_russian_roulette(ctx[g], rr)) return die("rr");
       if (pt_clear(ctx[g])) return die("clear");
     }
     auto t0 = std::chrono::steady_clock::now();
