@@ -16,10 +16,11 @@
 #include <cstring>
 #include <string>
 #include <algorithm>
+#include <array>
 #include <atomic>
 #include <chrono>
 #include <thread>
-#include <type_traits>
+#include <utility>
 #include <functional>
 #include <vector>
 
@@ -66,8 +67,6 @@ struct FiltGeom {
   int key, cls, geom;  // key = 2 * pair + half, as the scan reports its candidate
   float c[3], k[6], wk[6], ew_c, ew_w;
 };
-// launch-time variants of a bounce kernel: index nee | medium << 1 | glossy << 2 | roulette << 3 (variant_index)
-constexpr int kVariants = 16;
 struct pt_context {
   int device = 0;
   int sm_count = 0;
@@ -133,10 +132,9 @@ struct pt_context {
   float4* d_accum = nullptr;
   float* d_rgb = nullptr;      // staging for packed RGB
   uchar4* d_rgba8 = nullptr;   // staging for the 8-bit resolve
-  // persistent grid per (FIRST,LAST) slot and launch-time variant (variant_index); 0 = no such variant (NeeOf, MediumOf,
-  // GlossyOf, RouletteOf)
-  int grid_blocks[4][kVariants] = {};
-  int grid_blocks_q[2][kVariants] = {};  // k_bounce_q<LAST> (depths >= 1 of the linear mode)
+  // persistent grid of each entry of the kernel tables (kBounceKernels), 0 = no such kernel
+  int grid_blocks[2][2][kFxSets] = {};  // [FIRST][LAST][FX]: k_bounce, or k_bounce_bvh in the hierarchy mode
+  int grid_blocks_q[2][kFxSets] = {};   // [LAST][FX]: k_bounce_q (depths >= 1 of the linear mode)
   size_t q_smem_total = 0;            // k_bounce_q: filter geometry + the warps' candidate queues
   int q_mode = 0;                     // depths >= 1, few geoms: 0 = per depth by the scene's measured survival (h_policy),
                                       // 1 = always k_bounce_q, 2 = always the fused k_bounce (PT_B200_FUSED=1 / =0 force 2 / 1)
@@ -695,90 +693,51 @@ static RaygenConsts make_raygen(const pt_camera_data& c, const pt_lens* lens) {
   return R;
 }
 
-// the direct-light-sampling variant of (FIRST, LAST); the last segment never samples a light, and a first-and-last
-// segment cannot carry the no-emission flag either, so <true, true> needs no variant of its own
-template <bool F, bool L>
-struct NeeOf { static constexpr bool value = !(F && L); };
-// the subsurface-scattering variant of LAST: none for the last segment -- a scattering event there ends the path exactly as
-// the refraction it replaces does (neither adds radiance, and no later depth counts the path), so image and live counts
-// are those of the plain kernel
-template <bool L>
-struct MediumOf { static constexpr bool value = !L; };
-// the glossy-reflection variant of LAST: none, for the same reason -- the last segment stores no direction, so the
-// direction a glossy event samples there is never used
-template <bool L>
-struct GlossyOf { static constexpr bool value = !L; };
-// the Russian-roulette variant of (FIRST, LAST): none for the first segment, whose throughput is 1, nor for the last one,
-// which continues nowhere -- roulette runs at neither (DESIGN.md 4)
-template <bool F, bool L>
-struct RouletteOf { static constexpr bool value = !F && !L; };
-
-static int variant_index(bool nee, bool med, bool gl, bool rr) {
-  return (nee ? 1 : 0) | (med ? 2 : 0) | (gl ? 4 : 0) | (rr ? 8 : 0);
-}
-// Calls fn(N, M, G, R) with the launch-time switches (nee, med, gl, rr) of a bounce kernel of segment kind (F, L) as
-// std::bool_constant arguments: one instantiation per combination.  A switch the kind has no variant for (NeeOf,
-// MediumOf, GlossyOf, RouletteOf) is passed as false, so no instantiation is made that cannot be launched.
-template <bool F, bool L, typename Fn>
-static auto with_variant(bool nee, bool med, bool gl, bool rr, Fn&& fn) {
-  auto r = [&](auto N, auto M, auto G) {
-    return rr ? fn(N, M, G, std::bool_constant<RouletteOf<F, L>::value>{}) : fn(N, M, G, std::false_type{});
-  };
-  auto g = [&](auto N, auto M) { return gl ? r(N, M, std::bool_constant<GlossyOf<L>::value>{}) : r(N, M, std::false_type{}); };
-  auto m = [&](auto N) { return med ? g(N, std::bool_constant<MediumOf<L>::value>{}) : g(N, std::false_type{}); };
-  return nee ? m(std::bool_constant<NeeOf<F, L>::value>{}) : m(std::false_type{});
-}
-// a variant index whose switches segment kind (F, L) has a variant for
-template <bool F, bool L>
-static bool has_variant(int v) {
-  return ((v & 1) == 0 || NeeOf<F, L>::value) && ((v & 2) == 0 || MediumOf<L>::value) && ((v & 4) == 0 || GlossyOf<L>::value) &&
-         ((v & 8) == 0 || RouletteOf<F, L>::value);
+// The features the bounce kernels of segment kind (first, last) are instantiated with; a launch runs a subset of them.
+//   direct light sampling: unless first and last -- the last segment never samples a light, but it honours the
+//     no-emission flag, and a first-and-last segment cannot carry that flag either
+//   subsurface scattering: unless last -- a scattering event there ends the path exactly as the refraction it replaces
+//     does (neither adds radiance, and no later depth counts the path), so image and live counts are those of the plain
+//     kernel
+//   glossy reflection: unless last, for the same reason -- the last segment stores no direction, so the direction a
+//     glossy event samples there is never used
+//   Russian roulette: unless first, whose throughput is 1, or last, which continues nowhere (DESIGN.md 4)
+constexpr uint32_t variants_of(bool first, bool last) {
+  return (first && last ? 0u : kFxNee) | (last ? 0u : kFxMedium | kFxGlossy) | (first || last ? 0u : kFxRoulette);
 }
 
-// resident CTAs per SM of one bounce kernel with `smem` bytes of dynamic shared memory
-template <typename K>
-static int fit_kernel(K kernel, int threads, size_t smem, bool carveout, int* per_sm) {
+// The kernel tables: kBounceKernels[first][last][FX] holds the bounce kernels of that segment kind and feature set, null
+// where FX is not a subset of variants_of(first, last) -- no such kernel is instantiated.  (k_bounce_q and k_bounce_bvh
+// take no FIRST: the kinds (true, L) and (false, L) share their instantiations.)
+using BounceKernel = void (*)(BounceParams);
+struct BounceKernels {
+  BounceKernel fused, queued, bvh;  // k_bounce, k_bounce_q, k_bounce_bvh
+};
+template <bool F, bool L, uint32_t FX>
+constexpr BounceKernels bounce_kernels() {
+  if constexpr ((FX & ~variants_of(F, L)) != 0) return {nullptr, nullptr, nullptr};
+  else return {k_bounce<F, L, FX>, k_bounce_q<L, FX>, k_bounce_bvh<L, FX>};
+}
+template <bool F, bool L, uint32_t... FX>
+constexpr std::array<BounceKernels, kFxSets> kernel_table(std::integer_sequence<uint32_t, FX...>) {
+  return {{bounce_kernels<F, L, FX>()...}};
+}
+using EveryFx = std::make_integer_sequence<uint32_t, kFxSets>;
+static const std::array<BounceKernels, kFxSets> kBounceKernels[2][2] = {
+    {kernel_table<false, false>(EveryFx{}), kernel_table<false, true>(EveryFx{})},
+    {kernel_table<true, false>(EveryFx{}), kernel_table<true, true>(EveryFx{})}};
+
+// the persistent grid of one bounce kernel with `smem` bytes of dynamic shared memory: resident CTAs on the whole
+// device, 0 for a null table entry
+static int fit_grid(pt_context* c, BounceKernel kernel, int threads, size_t smem, bool carveout, const char* name, int* grid) {
+  *grid = 0;
+  if (!kernel) return PT_OK;
+  int per_sm = 0;
   CU(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   if (carveout) CU(cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-  CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(per_sm, kernel, threads, smem));
-  return PT_OK;
-}
-
-template <bool F, bool L>
-static int setup_variant(pt_context* c, int slot) {
-  for (int v = 0; v < kVariants; v++) {
-    c->grid_blocks[slot][v] = 0;
-    if (!has_variant<F, L>(v)) continue;
-    int per_sm = 0;
-    // (many geoms: one kernel for every depth, primary rays come from k_raygen_wf)
-    const int rc = with_variant<F, L>(v & 1, v & 2, v & 4, v & 8, [&](auto N, auto M, auto G, auto R) {
-      constexpr bool n = decltype(N)::value, m = decltype(M)::value, g = decltype(G)::value, r = decltype(R)::value;
-      return c->mode ? fit_kernel(k_bounce_bvh<L, n, m, g, r>, kBvhThreads, kBvhSmemBytes, false, &per_sm)
-                     : fit_kernel(k_bounce<F, L, n, m, g, r>, kBounceThreads, c->smem_bytes, false, &per_sm);
-    });
-    if (rc) return rc;
-    if (per_sm < 1) { pt_set_error_("k_bounce does not fit on an SM"); return PT_ERR_CUDA; }
-    c->grid_blocks[slot][v] = per_sm * c->sm_count;
-  }
-  return PT_OK;
-}
-
-// (the last segment never samples a light, but it honours the no-emission flag: k_bounce_q<true> has NEE variants --
-// NeeOf<false, L>)
-template <bool L>
-static int setup_variant_q(pt_context* c, int slot) {
-  for (int v = 0; v < kVariants; v++) {
-    c->grid_blocks_q[slot][v] = 0;
-    if (!has_variant<false, L>(v)) continue;
-    int per_sm = 0;
-    const int rc = with_variant<false, L>(v & 1, v & 2, v & 4, v & 8, [&](auto N, auto M, auto G, auto R) {
-      return fit_kernel(k_bounce_q<L, decltype(N)::value, decltype(M)::value, decltype(G)::value, decltype(R)::value>, kQThreads,
-                        c->q_smem_total, true, &per_sm);
-    });
-    if (rc) return rc;
-    if (per_sm < 1) { pt_set_error_("k_bounce_q does not fit on an SM"); return PT_ERR_CUDA; }
-    c->grid_blocks_q[slot][v] = per_sm * c->sm_count;
-  }
+  CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, threads, smem));
+  if (per_sm < 1) { pt_set_error_("%s does not fit on an SM", name); return PT_ERR_CUDA; }
+  *grid = per_sm * c->sm_count;
   return PT_OK;
 }
 
@@ -1056,16 +1015,17 @@ static int upload_scene(pt_context* c, const pt_static_geom* geoms, int n_geoms,
     c->geom_smem = filt_smem_bytes(cap);
     c->mode = mode;
     c->smem_bytes = mode == 0 ? c->geom_smem : kBvhSmemBytes;  // k_bounce: filter geometry; k_bounce_bvh: pool results, retry list, stacks
-    int rc;
-    if ((rc = setup_variant<true, false>(c, 0))) return rc;
-    if ((rc = setup_variant<true, true>(c, 1))) return rc;
-    if ((rc = setup_variant<false, false>(c, 2))) return rc;
-    if ((rc = setup_variant<false, true>(c, 3))) return rc;
-    if (mode == 0) {
-      c->q_smem_total = c->geom_smem + q_smem_bytes();
-      if ((rc = setup_variant_q<false>(c, 0))) return rc;
-      if ((rc = setup_variant_q<true>(c, 1))) return rc;
-    }
+    if (mode == 0) c->q_smem_total = c->geom_smem + q_smem_bytes();
+    for (int f = 0; f < 2; f++)
+      for (int l = 0; l < 2; l++)
+        for (uint32_t fx = 0; fx < kFxSets; fx++) {
+          const BounceKernels& k = kBounceKernels[f][l][fx];
+          // (many geoms: one kernel for every depth, primary rays come from k_raygen_wf)
+          int rc = mode ? fit_grid(c, k.bvh, kBvhThreads, kBvhSmemBytes, false, "k_bounce", &c->grid_blocks[f][l][fx])
+                        : fit_grid(c, k.fused, kBounceThreads, c->smem_bytes, false, "k_bounce", &c->grid_blocks[f][l][fx]);
+          if (!rc && mode == 0 && !f) rc = fit_grid(c, k.queued, kQThreads, c->q_smem_total, true, "k_bounce_q", &c->grid_blocks_q[l][fx]);
+          if (rc) return rc;
+        }
     CU(cudaFuncSetAttribute(k_intersect_list, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c->geom_smem));
     CU(cudaFuncSetAttribute(k_primary_list, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c->geom_smem));
   }
@@ -1254,44 +1214,42 @@ extern "C" int pt_clear(pt_context* c) {
   return PT_OK;
 }
 
-template <bool F, bool L>
-static cudaError_t launch_bounce(pt_context* c, int slot, const BounceParams& P, uint32_t n_upper, cudaStream_t st) {
-  const bool nee = c->nee && c->n_lights > 0 && NeeOf<F, L>::value;
-  const bool med = MediumOf<L>::value && c->sss && c->n_media > 0;  // (no medium in the scene: the plain kernels, same results)
-  const bool gl = GlossyOf<L>::value && c->glossy && c->n_glossy > 0;  // (likewise without a glossy geom)
-  const bool rr = RouletteOf<F, L>::value && c->rr_first > 0 && P.depth >= (uint32_t)c->rr_first;  // (a roulette depth)
-  const int v = variant_index(nee, med, gl, rr);
-  uint32_t grid = (uint32_t)c->grid_blocks[slot][v];
+// the features a launch at `depth` runs: those switched on that the scene has a use for, roulette from its first depth
+// on, and only those its segment kind has variants for
+static uint32_t launch_features(const pt_context* c, bool first, bool last, uint32_t depth) {
+  uint32_t fx = 0;
+  if (c->nee && c->n_lights > 0) fx |= kFxNee;
+  if (c->sss && c->n_media > 0) fx |= kFxMedium;  // (no medium in the scene: the plain kernels, same results)
+  if (c->glossy && c->n_glossy > 0) fx |= kFxGlossy;  // (likewise without a glossy geom)
+  if (c->rr_first > 0 && depth >= (uint32_t)c->rr_first) fx |= kFxRoulette;  // (a roulette depth)
+  return fx & variants_of(first, last);
+}
+
+static cudaError_t launch_bounce(pt_context* c, bool first, bool last, const BounceParams& P, uint32_t n_upper, cudaStream_t st) {
+  const uint32_t fx = launch_features(c, first, last, P.depth);
+  const BounceKernels& k = kBounceKernels[first][last][fx];
+  uint32_t grid = (uint32_t)c->grid_blocks[first][last][fx];
   // depths >= 1, few geoms: second half re-batched by winner type -- unless the scene keeps nearly all its paths alive
   // at this depth (closed rooms), where the fused kernel is faster; unknown yet (first wavefronts of a scene): re-batched
   const bool use_q = c->q_mode == 1 || (c->q_mode == 0 && ((volatile int*)c->h_policy)[P.depth] != 2);
-  if (!F && !c->mode && use_q) {
-    uint32_t gq = (uint32_t)c->grid_blocks_q[L ? 1 : 0][v];
+  if (!first && !c->mode && use_q) {
+    uint32_t gq = (uint32_t)c->grid_blocks_q[last][fx];
     const uint32_t ctas = (n_upper + kQThreads - 1) / kQThreads;  // one unit per warp at least
     if (ctas < gq) gq = ctas ? ctas : 1;
-    with_variant<F, L>(nee, med, gl, rr, [&](auto N, auto M, auto G, auto R) {
-      k_bounce_q<L, decltype(N)::value, decltype(M)::value, decltype(G)::value, decltype(R)::value>
-          <<<gq, kQThreads, c->q_smem_total, st>>>(P);
-    });
+    k.queued<<<gq, kQThreads, c->q_smem_total, st>>>(P);
   } else if (c->mode) {
-    if (F) {  // primary rays into the wavefront's input buffers
+    if (first) {  // primary rays into the wavefront's input buffers
       const uint32_t blocks = (n_upper + 255u) / 256u, most = (uint32_t)c->sm_count * 8u;
       k_raygen_wf<<<blocks < most ? (blocks ? blocks : 1u) : most, 256, 0, st>>>(P);
       c->launches++;
     }
     const uint32_t ctas = (n_upper + kPoolMin * (kBvhThreads / 32) - 1) / (kPoolMin * (kBvhThreads / 32));  // a (smallest) pool per warp at least
     if (ctas < grid) grid = ctas ? ctas : 1;
-    with_variant<F, L>(nee, med, gl, rr, [&](auto N, auto M, auto G, auto R) {
-      k_bounce_bvh<L, decltype(N)::value, decltype(M)::value, decltype(G)::value, decltype(R)::value>
-          <<<grid, kBvhThreads, kBvhSmemBytes, st>>>(P);
-    });
+    k.bvh<<<grid, kBvhThreads, kBvhSmemBytes, st>>>(P);
   } else {
     const uint32_t ctas = (n_upper + kBounceThreads - 1) / kBounceThreads;  // one unit per warp at least
     if (ctas < grid) grid = ctas ? ctas : 1;
-    with_variant<F, L>(nee, med, gl, rr, [&](auto N, auto M, auto G, auto R) {
-      k_bounce<F, L, decltype(N)::value, decltype(M)::value, decltype(G)::value, decltype(R)::value>
-          <<<grid, kBounceThreads, c->smem_bytes, st>>>(P);
-    });
+    k.fused<<<grid, kBounceThreads, c->smem_bytes, st>>>(P);
   }
   c->launches++;
   return cudaGetLastError();
@@ -1416,11 +1374,7 @@ static int render_into(pt_context* c, uint32_t first_sample, uint32_t n_samples,
       P.cap = (uint32_t)cap;
       P.ptab = c->ptab_on ? c->d_ptab : nullptr;
       const bool first = depth == 0, last = depth == max_depth - 1;
-      cudaError_t e;
-      if (first && last) e = launch_bounce<true, true>(c, 1, P, n_first, st);
-      else if (first) e = launch_bounce<true, false>(c, 0, P, n_first, st);
-      else if (last) e = launch_bounce<false, true>(c, 3, P, n_first, st);
-      else e = launch_bounce<false, false>(c, 2, P, n_first, st);
+      cudaError_t e = launch_bounce(c, first, last, P, n_first, st);
       if (e != cudaSuccess) { pt_set_error_("k_bounce launch failed: %s", cudaGetErrorString(e)); return PT_ERR_CUDA; }
       // direct light sampling: the shadow rays this depth queued, before the next depth queues its own
       if (nee_on && !last && (e = launch_shadow(c, P, n_first, st)) != cudaSuccess) {
